@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
   python bench.py --impl reference [--steps K] [--warmup W]      # the reference's own kernels on the host cores
+  python bench.py ... --dump-outputs DIR                         # + what the last timed step computed, DIR/<name>.npy
 
 A step = one full training iteration of the per-ray hot path on one batch of 8192 synthetic rays per GPU:
 sample (octree traversal + march) -> hash encode -> MLP -> composite -> Charbonnier -> backward of all of it
@@ -403,6 +404,8 @@ def render_arm(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rgb": rgb, "depth": depth, "accumulation": acc})
     emit(({
         "metric": "render rays/sec (forward only), 1920x1080 frames, log2T=23", "value": W * H / (ms * 1e-3),
         "unit": "rays/s", "n_gpus": 1, "steps": steps, "warmup": warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -470,6 +473,33 @@ def operator_api_arm(rig, dev, steps, warmup, hidden, log2t):
                     "+ torch.optim.Adam: the drop-in for gfnerf/nerfacto.py:522-619 under nerfstudio's trainer"}
 
 
+DUMP_TABLE_SAMPLE = 1 << 20     # hash-table entries in the dump (a fixed, seeded sample of the 16.8 M)
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy, float32 (float64 for integers), so that two builds of the project can be
+    compared output for output on the same inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        a = a.astype(np.float64 if a.dtype.kind in "iub" else np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def step_arrays(out, eng):
+    """What a caller of the training step receives (GFNeRFEngine.train_step's StepOutputs) and the model's parameters
+    after it: MLPs, appearance embedding and a seeded sample of the hash table (the whole table is 64 MB of fp32)."""
+    import torch
+    table = eng.enc.feat_pool_.detach().reshape(-1)
+    pick = torch.from_numpy(np.sort(np.random.RandomState(0).choice(table.numel(), min(DUMP_TABLE_SAMPLE, table.numel()),
+                                                                    replace=False))).to(table.device)
+    arrays = {"rgb": out.rgb, "depth": out.depth, "accumulation": out.accumulation, "loss": out.loss,
+              "n_samples": out.n_samples, "mlp_params": eng.mlp, "hash_table_sample": table[pick]}
+    if eng.emb is not None:
+        arrays["appearance_embedding"] = eng.emb
+    return arrays
+
+
 # --------------------------------------------------------------------------------------------
 _REAL_STDOUT = None
 
@@ -507,10 +537,15 @@ def main():
                          "one private residual sub-encoder per GPU (log2T 21), no gradient exchange.  render: config 5 "
                          "-- forward-only 1920x1080 frames, log2T 23, eval sampling; a step = one frame")
     ap.add_argument("--breakdown", action="store_true", help="print the per-kernel table to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, "
+                         "seeded inputs: the same arguments give the same inputs on every run)")
     ap.add_argument("--hidden", type=int, default=64, choices=[64, 128],
                     help="MLP width: 64 = the north star's / nerfstudio's default (the bench line); 128 = the "
                          "reference's shipped gf-nerf config (gfnerf/config.py:124-125)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "reference":
         reference_arm(args)
         return
@@ -589,7 +624,7 @@ def main():
         e0.record()
         t_host = time.perf_counter()
         for i in range(steps):
-            fn(warmup + i)
+            out = fn(warmup + i)
         host_ms.append((time.perf_counter() - t_host) * 1e3 / steps)   # host time to ENQUEUE a step (no sync inside)
         eng.flush()            # the last step's (deferred, N > 1) optimizer step belongs to the timed region
         e1.record()
@@ -600,18 +635,20 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t)
-        return ms, launches
+        return ms, launches, out
 
     clocks = ClockSampler(local)
     if not os.environ.get("GF_NO_CLOCKS"):      # (A/B: does polling nvidia-smi perturb the timed region?)
         clocks.start()
     if os.environ.get("GF_MAIN_PRIO"):      # A/B: run the step on a non-default stream of the given priority
         torch.cuda.set_stream(torch.cuda.Stream(device=dev, priority=int(os.environ["GF_MAIN_PRIO"])))
-    ms_total, launches = timed(step_resident, args.steps, args.warmup)
+    ms_total, launches, last = timed(step_resident, args.steps, args.warmup)
     clocks.stop_flag = True
+    if args.dump_outputs and rank == 0:   # before the next leg's steps reuse the output buffers and move the parameters
+        dump_outputs(args.dump_outputs, step_arrays(last, eng))
     ms_step = ms_total / args.steps
     value = RAYS_PER_GPU * world * args.steps / (ms_total * 1e-3)
-    ms_e2e, _ = timed(step_e2e, args.steps, 3)       # the loss copies are stream-ordered: inside the timed region
+    ms_e2e, _, _ = timed(step_e2e, args.steps, 3)       # the loss copies are stream-ordered: inside the timed region
     e2e_losses = eng.read_losses()
     assert len(e2e_losses) == args.steps + 3 and all(np.isfinite(e2e_losses)), e2e_losses
     e2e_value = RAYS_PER_GPU * world * args.steps / (ms_e2e * 1e-3)

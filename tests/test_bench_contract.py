@@ -62,3 +62,23 @@ def test_cpu_arm_falls_back_to_the_port_and_says_so(monkeypatch):
     monkeypatch.setattr(bench, "time_reference_native", boom)
     out = bench.time_cpu_arm(8, 1, 0)
     assert out[4] == "port" and "OSError" in out[5]
+
+
+@pytest.mark.gpu
+@pytest.mark.timeout(900)
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """--dump-outputs: the arrays of the last timed step as float32 / float64 .npy files, 64 MB at most, and the JSON
+    line still the only stdout."""
+    import numpy as np
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--no-operator-api", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, cwd=ROOT, timeout=880)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert len([l for l in r.stdout.splitlines() if l.strip()]) == 1 and json.loads(r.stdout)["steps"] == 2
+    files = {p.name: np.load(p) for p in out.iterdir()}
+    assert {"rgb.npy", "depth.npy", "accumulation.npy", "loss.npy", "mlp_params.npy", "hash_table_sample.npy"} <= set(files)
+    assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+    assert sum(p.stat().st_size for p in out.iterdir()) <= 64 << 20
+    assert files["rgb.npy"].shape == (8192, 3) and np.isfinite(files["rgb.npy"]).all()
+    assert np.isfinite(files["loss.npy"]).all() and files["n_samples.npy"][0] > 0

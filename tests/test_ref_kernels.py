@@ -446,45 +446,46 @@ def test_cuda_sampler_counts_and_anchors_are_the_reference_kernels(fx, rig, mode
 
 
 # ------------------------------------------------------------------ GPU: beside the reference's kernels built by nvcc
-# `make -C oracle ref_cuda` (build container; the .so travels to the GPU box).  Runs whenever that library exists.
-# The bit-level pin the host build cannot give: nvcc's own FMA contraction of the reference's expressions.  First run
-# (r02a, profiles/r02a_ref_cuda.log): hash forward, counts, anchors, first_oct_dis identical; t / warp differed in the
-# last bits through two contractions read off the reference's SASS and now followed by kernel + oracle (the GEMV's
-# rounded product is the second one; the leaf-crossing step is fused into `cur_t +=`).
-ref_cuda = pytest.mark.skipif(not rh.cuda_available(), reason="needs oracle/_ref/libgf_ref_cuda.so")
+# `make -C oracle ref_cuda` (needs the reference's source tree).  The bit-level pin the host build cannot give: nvcc's own
+# FMA contraction of the reference's expressions.  First run (r02a, profiles/r02a_ref_cuda.log): hash forward, counts,
+# anchors, first_oct_dis identical; t / warp differed in the last bits through two contractions read off the
+# reference's SASS and now followed by kernel + oracle (the GEMV's rounded product is the second one; the leaf-crossing
+# step is fused into `cur_t +=`).  Where that library is not built, a seeded sample of the same outputs stored in
+# tests/golden/ref_cuda.npz stands in for it (tests/golden/make_golden_ref_cuda.py).
+REF_CUDA_GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_cuda.npz")
 
 
-@pytest.mark.gpu
-@ref_cuda
-def test_cuda_beside_the_reference_kernels_built_by_nvcc(rig):
+def beside_nvcc_inputs(rig):
+    """The inputs of the comparison with the nvcc-built reference kernels: a hash-encoding batch along rays and a
+    sampler batch of 4096 rig rays (unit directions) with its march noise."""
+    from gfnerf_b200.persoctree import rig_rays
+    feat, prim, bias, pts, anchors = hash_inputs(200000, 7, 16, seed=3, along_rays=True)
+    R = 4096
+    o, d, _ = rig_rays(rig["c2w"], rig["intri"], R, seed=77)
+    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(np.float32)
+    noise = np.random.RandomState(5).uniform(0.5, 1.5, S + R + 10).astype(np.float32)
+    return dict(feat=feat, prim=prim, bias=bias, pts=pts, anchors=anchors, o=o, d=d, noise=noise)
+
+
+def cuda_beside_nvcc(rig, inp):
+    """gf_hash_forward and the sampler's launch on `beside_nvcc_inputs` -> (sampler, dict of device tensors)"""
     import torch
     from gfnerf_b200 import _lib
-    from gfnerf_b200.persoctree import rig_rays
     from tests.helpers import make_sampler
     dev = "cuda"
     T = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
-    # hash forward: same table, points, primes -> bit-identical encodings
-    feat, prim, bias, pts, anchors = hash_inputs(200000, 7, 16, seed=3, along_rays=True)
+    feat, prim, bias, pts, anchors = (inp[k] for k in ("feat", "prim", "bias", "pts", "anchors"))
     L = feat.shape[0] // 16
-    ref = rh.cuda_hash_forward(T(feat), T(prim.astype(np.int32)), T(bias), T(pts), T(anchors))
     scales_d, scales_h = torch.empty(16, device=dev), np.zeros(16, np.float32)
     _lib.check(_lib.lib().gf_hash_level_scales(_lib.ptr(scales_d), scales_h.ctypes.data, _lib.cur_stream()))
     f16 = T(feat).half().contiguous()
     tp, ta, tprim, tbias = T(pts), T(anchors), T(prim.astype(np.int32)), T(bias)
-    out = torch.empty((pts.shape[0], 32), device=dev)
-    _lib.check(_lib.lib().gf_hash_forward(pts.shape[0], None, 7, L, _lib.ptr(f16), _lib.ptr(tprim), _lib.ptr(tbias),
-                                          _lib.ptr(scales_d), _lib.ptr(tp), _lib.ptr(ta), 1, None, _lib.ptr(out),
-                                          _lib.cur_stream()))
-    torch.cuda.synchronize()
-    print("hash forward bit-equal fraction vs nvcc-built reference:", float((out == ref).float().mean()))
-    assert torch.equal(out, ref)
-    # sampler: leaf ranges, counts and anchors identical; positions reported
+    hash_out = torch.empty((pts.shape[0], 32), device=dev)
+    _lib.check(_lib.lib().gf_hash_forward(pts.shape[0], None, prim.shape[1], L, _lib.ptr(f16), _lib.ptr(tprim),
+                                          _lib.ptr(tbias), _lib.ptr(scales_d), _lib.ptr(tp), _lib.ptr(ta), 1, None,
+                                          _lib.ptr(hash_out), _lib.cur_stream()))
     s = make_sampler(rig, mode=1)
-    R = 4096
-    o, d, _ = rig_rays(rig["c2w"], rig["intri"], R, seed=77)
-    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(np.float32)
-    noise = T(np.random.RandomState(5).uniform(0.5, 1.5, S + R + 10).astype(np.float32))
-    r = rh.cuda_get_samples(T(o), T(d), noise, s.tree_nodes_gpu_, s.pers_trans_gpu_, T(orc.search_order()))
+    R = inp["o"].shape[0]
     z = lambda *sh, dt=torch.float32: torch.zeros(sh, dtype=dt, device=dev)
     world, warp, dirs, anc = z(R, S, 3), z(R, S, 3), z(R, S, 3), z(R, S, 3, dt=torch.int64)
     dists, ts, se, first, cnt = z(R, S), z(R, S), z(R, 2, dt=torch.int64), z(R, 1), z(R, dt=torch.int32)
@@ -492,10 +493,43 @@ def test_cuda_beside_the_reference_kernels_built_by_nvcc(rig):
                          dists=_lib.ptr(dists), ts=_lib.ptr(ts), anchors_i64=_lib.ptr(anc), anchors_i32=None,
                          pts_idx_start_end=_lib.ptr(se), counts=_lib.ptr(cnt), first_oct_dis=_lib.ptr(first),
                          n_oct=None, packed=None)
-    s._launch(T(o), T(d), noise, so)
+    s._launch(T(inp["o"]), T(inp["d"]), T(inp["noise"]), so)
     torch.cuda.synchronize()
+    return s, dict(hash_out=hash_out, counts=cnt, first_oct_dis=first.view(-1), ts=ts, dists=dists, warp_pts=warp,
+                   world_pts=world, anchors=anc)
+
+
+@pytest.mark.gpu
+def test_cuda_beside_the_reference_kernels_built_by_nvcc(rig):
+    import torch
+    inp = beside_nvcc_inputs(rig)
+    s, got = cuda_beside_nvcc(rig, inp)
+    # the stored sample: every value bit for bit (hash rows, per-ray counts and first crossings, the samples of the
+    # stored rays)
+    gold = np.load(REF_CUDA_GOLD)
+    h = lambda k: got[k].cpu().numpy()
+    assert np.array_equal(h("hash_out")[gold["hash_rows"]], gold["hash_out"])
+    assert np.array_equal(h("counts"), gold["counts"]) and np.array_equal(h("first_oct_dis"), gold["first_oct_dis"])
+    rays = gold["rays"]
+    m = np.arange(S)[None, :] < gold["counts"][rays][:, None]
+    for k in ("ts", "dists", "warp_pts", "world_pts", "anchors"):
+        assert np.array_equal(h(k)[rays][m], gold[k]), k
+    if not rh.cuda_available():
+        return
+    # live, beside the library: hash forward on the same table, points, primes -> bit-identical encodings
+    dev = "cuda"
+    T = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+    ref = rh.cuda_hash_forward(T(inp["feat"]), T(inp["prim"].astype(np.int32)), T(inp["bias"]), T(inp["pts"]),
+                               T(inp["anchors"]))
+    out = got["hash_out"]
+    print("hash forward bit-equal fraction vs nvcc-built reference:", float((out == ref).float().mean()))
+    assert torch.equal(out, ref)
+    # sampler: leaf ranges, counts and anchors identical; positions reported
+    r = rh.cuda_get_samples(T(inp["o"]), T(inp["d"]), T(inp["noise"]), s.tree_nodes_gpu_, s.pers_trans_gpu_,
+                            T(orc.search_order()))
+    cnt, ts, dists, warp, world, anc = (got[k] for k in ("counts", "ts", "dists", "warp_pts", "world_pts", "anchors"))
     same = (cnt == r["counts"])
-    print("sampler: rays with identical sample counts:", float(same.float().mean()), "of", R)
+    print("sampler: rays with identical sample counts:", float(same.float().mean()), "of", cnt.shape[0])
     m = (torch.arange(S, device=dev)[None, :] < cnt[:, None]) & same[:, None]
     for name, a, b in (("t", ts, r["ts"]), ("dist", dists, r["dists"]), ("warp", warp, r["warp_pts"]),
                        ("world", world, r["world_pts"])):
@@ -504,7 +538,7 @@ def test_cuda_beside_the_reference_kernels_built_by_nvcc(rig):
               f"max abs diff {float((a[mm] - b[mm]).abs().max()):.3e}")
     assert bool(same.all())
     assert torch.equal(anc[m], r["anchors"][m])
-    assert torch.equal(first.view(-1), r["first_oct_dis"])
+    assert torch.equal(got["first_oct_dis"], r["first_oct_dis"])
     for a, b in ((ts, r["ts"]), (dists, r["dists"]), (warp, r["warp_pts"]), (world, r["world_pts"])):
         mm = m if a.dim() == 2 else m[..., None].expand_as(a)
         assert torch.equal(a[mm], b[mm])
