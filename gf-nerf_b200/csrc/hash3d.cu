@@ -19,8 +19,6 @@
 //    vectorised fp32 reductions (red.global.add.v2.f32) once (hash_common.cuh).
 //
 // Arithmetic follows the oracle's FMA convention exactly (oracle/gf_oracle.c).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "hash_common.cuh"
 
@@ -50,7 +48,7 @@ __global__ void cast_table_tail_kernel(const float* __restrict__ in, __half* __r
 }
 
 constexpr int kHashBlock = 256;
-// Two register / scheduling variants of the forward gather (tools/hash_variants.py, r02u, bench samples):
+// Two register / scheduling variants of the forward gather (r02u, bench samples), chosen by hash_forward_impl:
 //   PREFETCH = false  48 registers, 5 CTAs per SM: the most warps in flight -- best when the table does not fit the
 //                     L2 and the gather waits on HBM (log2T = 23: 1.79 ms against 2.15 for the other one);
 //   PREFETCH = true   the 32 gathers of a four-level group are all issued before the first is consumed, 79 registers,
@@ -151,7 +149,7 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
                 const int32_t* __restrict__ prim_pool, const float* __restrict__ bias_pool,
                 const float* __restrict__ scales, const float* __restrict__ pts,
                 const AnchorT* __restrict__ anchors, const void* __restrict__ grad_in_v,
-                float* __restrict__ grad_table, int aggregate, int level_begin, int level_end) {
+                float* __restrict__ grad_table, int level_begin, int level_end) {
   if (d_n_ptr) {
     int64_t dn = *d_n_ptr;
     n = dn < n ? dn : n;
@@ -209,7 +207,7 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
         }
       }
       hash_scatter_level<POW2, HAS_BIAS, UNSCALE>(l, x, y, z, vol, valid, gh, lane, n_volumes, local_size, prim_pool,
-                                                  bias_pool, s_scale[l], grad_table, aggregate,
+                                                  bias_pool, s_scale[l], grad_table,
                                                   s_stage + (threadIdx.x >> 5) * kScatterWarpWords);
     }
   }
@@ -289,9 +287,7 @@ static int hash_forward_impl(int64_t n, const int32_t* d_n_ptr, int32_t n_volume
   const int grid = stride_grid(n, kHashBlock, 8, 4);
   const bool p2 = is_pow2(local_size);
   // the rows the levels can reach (8.5 * local_size, 4 bytes each) against the 126 MB L2: which variant (see the kernel)
-  // GF_HASH_FWD_VARIANT = 0 / 1 forces one (A/B measurements, tools/hash_variants.py)
-  static const int forced = [] { const char* e = getenv("GF_HASH_FWD_VARIANT"); return e ? atoi(e) : -1; }();
-  const bool l2_resident = forced >= 0 ? forced != 0 : (int64_t)local_size * 34 <= (int64_t)100 << 20;
+  const bool l2_resident = (int64_t)local_size * 34 <= (int64_t)100 << 20;
 #define GF_FWD_V(P2, AT, O16, O32, PF)                                                                        \
   hash_fwd_kernel<P2, AT, O16, O32, PF><<<grid, kHashBlock, 0, st>>>(                                         \
       n, d_n_ptr, n_volumes, (uint32_t)local_size, (const __half2*)feat_f16, prim_pool, bias_pool,            \
@@ -360,14 +356,11 @@ int gf_hash_backward_levels(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = stride_grid(n, kHashBlock, 4, 4);
   const bool p2 = is_pow2(local_size);
-  // Run aggregation: 0 = off (every lane scatters on its own; profiling A/B only), n > 0 = runs of up to n lanes go
-  // through the segmented shuffle reduction, longer ones through shared memory.  GF_HASH_AGG overrides (A/B).
-  static const int aggregate = [] { const char* e = getenv("GF_HASH_AGG"); return e ? atoi(e) : 4; }();
   const bool g16 = (grad_in_is_scaled_f16 & 1) != 0, unscale = (grad_in_is_scaled_f16 & 2) == 0;
 #define GF_BWD(P2, AT, G16, HB, US)                                                                              \
   hash_bwd_kernel<P2, AT, G16, HB, US><<<grid, kHashBlock, 0, st>>>(n, d_n_ptr, n_volumes, (uint32_t)local_size, \
                                                                     prim_pool, bias_pool, level_scales, pts,     \
-                                                                    (const AT*)anchors, grad_in, grad_table, aggregate,  \
+                                                                    (const AT*)anchors, grad_in, grad_table,     \
                                                                     level_begin, level_end)
 #define GF_BWD_U(P2, AT, G16, HB)                  \
   do {                                             \

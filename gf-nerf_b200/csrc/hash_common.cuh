@@ -83,6 +83,8 @@ __device__ __forceinline__ void weights(const Cell& c, float (&w)[8]) {
 // wavefronts per warp and level with float2 contributions and separate rows -> 16 + 16.)
 constexpr int kScatterRowWords = 18;
 constexpr int kScatterWarpWords = 32 * kScatterRowWords;
+// longest run of lanes the segmented shuffle reduction takes; longer runs go through shared memory
+constexpr int kScatterShuffleMaxRun = 4;
 
 // red.global.add.v2.f32 of (s0, s1) * out_scale to tab[row] unless both are zero or `mask` (0 / ~0) is off: one
 // predicated instruction, no branch and no reconvergence bookkeeping around the 8 corner updates of a level
@@ -130,7 +132,7 @@ __device__ __forceinline__ void red_add_f32x2(const char* tab, uint32_t row, flo
 // fp16, one F2FP per corner), then add them to the fp32 gradient table.  Lanes that fall into the same cell of the
 // same volume (contiguous runs along the ray) are summed first; three warp-uniform paths by the longest run:
 //   1        every lane issues its own 8 predicated vector reductions;
-//   2..4     segmented shuffle reduction (1-2 steps), the run's first lane issues the reductions;
+//   2..4     segmented shuffle reduction (1-2 steps, kScatterShuffleMaxRun), the run's first lane issues the reductions;
 //   > 4      the contributions and rows go through shared memory and lane (corner d = lane & 7, quarter q = lane >> 3)
 //            walks the 8 rows of its quarter in lane order, flushing its fp32 partial sum at every run boundary:
 //            8 loads + 16 adds per lane whatever the run structure (a 5-step shuffle tree costs 80 + 80).
@@ -142,8 +144,7 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
                                                    int lane, int32_t n_volumes, uint32_t local_size,
                                                    const int32_t* __restrict__ prim_pool,
                                                    const float* __restrict__ bias_pool, float scale,
-                                                   float* __restrict__ grad_table, int aggregate,
-                                                   float* __restrict__ s_warp) {
+                                                   float* __restrict__ grad_table, float* __restrict__ s_warp) {
   const int tr = (l * n_volumes + vol) * 3;
   const Cell c = cell_of(x, y, z, scale, HAS_BIAS ? bias_pool + tr : nullptr);
   const uint32_t pa = (uint32_t)__ldg(prim_pool + tr), pb = (uint32_t)__ldg(prim_pool + tr + 1),
@@ -161,20 +162,15 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
     cq[d] = *reinterpret_cast<const uint32_t*>(&h);
   }
   const char* tab = reinterpret_cast<const char*>(grad_table) + (uint64_t)level_base_row(l, local_size) * 8u;
-  int maxrun = 1;
-  uint32_t heads = 0xffffffffu;
-  int end = lane + 1;
-  if (aggregate) {
-    const uint32_t ppx = __shfl_up_sync(0xffffffffu, c.px, 1), ppy = __shfl_up_sync(0xffffffffu, c.py, 1),
-                   ppz = __shfl_up_sync(0xffffffffu, c.pz, 1);
-    const int pvol = __shfl_up_sync(0xffffffffu, vol, 1);
-    const bool head = lane == 0 || ppx != c.px || ppy != c.py || ppz != c.pz || pvol != vol;
-    heads = __ballot_sync(0xffffffffu, head);
-    const uint32_t above = lane == 31 ? 0u : (heads & (0xffffffffu << (lane + 1)));
-    end = above ? (__ffs(above) - 1) : 32;
-    maxrun = (int)__reduce_max_sync(0xffffffffu, head ? (unsigned)(end - lane) : 0u);
-  }
-  if (maxrun > aggregate) {  // warp-uniform; aggregate = longest run the shuffle path still takes (4)
+  const uint32_t ppx = __shfl_up_sync(0xffffffffu, c.px, 1), ppy = __shfl_up_sync(0xffffffffu, c.py, 1),
+                 ppz = __shfl_up_sync(0xffffffffu, c.pz, 1);
+  const int pvol = __shfl_up_sync(0xffffffffu, vol, 1);
+  const bool head = lane == 0 || ppx != c.px || ppy != c.py || ppz != c.pz || pvol != vol;
+  const uint32_t heads = __ballot_sync(0xffffffffu, head);
+  const uint32_t above = lane == 31 ? 0u : (heads & (0xffffffffu << (lane + 1)));
+  const int end = above ? (__ffs(above) - 1) : 32;
+  const int maxrun = (int)__reduce_max_sync(0xffffffffu, head ? (unsigned)(end - lane) : 0u);
+  if (maxrun > kScatterShuffleMaxRun) {  // warp-uniform
     uint2* row = reinterpret_cast<uint2*>(s_warp + lane * kScatterRowWords);
 #pragma unroll
     for (int d = 0; d < 8; d++) row[d] = make_uint2(cq[d], pos[d]);

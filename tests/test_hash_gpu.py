@@ -3,9 +3,12 @@
 Bar: bit-exact corner rows and bit-exact forward values (both follow the same FMA convention);
 gradients within 1e-5 relative of the exactly-summed oracle (fp32 atomics, order-dependent).
 """
+import re
+
 import numpy as np
 import pytest
 import torch
+from torch.profiler import ProfilerActivity, profile
 
 from oracle import oracle as orc
 from tests.helpers import hash_inputs
@@ -32,8 +35,14 @@ def test_device_level_scales_reported():
     print("device exp2f level scales bit-equal to host:", bool(np.array_equal(dev, host)))
 
 
+def fwd_prefetch_args(prof):
+    """the PREFETCH template argument (the last one) of every hash_fwd_kernel instantiation a profile recorded"""
+    return {m.group(1) for e in prof.key_averages() for m in re.finditer(r"hash_fwd_kernel<[^>]*, (\w+)>", e.key)}
+
+
 # the last three: the table sizes of BASELINE.json configs[1] (global stage, log2T = 19), configs[3] (focal stage, 21) and
-# configs[4] (render, 23) -- value-level parity at the sizes the bench runs, on as many points as the oracle does in seconds
+# configs[4] (render, 23) -- value-level parity at the sizes the bench runs, on as many points as the oracle does in
+# seconds, and both gather variants: the prefetching one while the reachable rows fit the L2 (up to 21), the other at 23
 @pytest.mark.parametrize("n,n_vol,log2T,along", [(4096, 5, 12, True), (10000, 37, 15, False), (33, 1, 4, True),
                                                  (16384, 37, 19, True), (8192, 37, 21, True), (4096, 37, 23, False)])
 def test_corner_rows_and_forward_bit_exact(n, n_vol, log2T, along):
@@ -48,12 +57,15 @@ def test_corner_rows_and_forward_bit_exact(n, n_vol, log2T, along):
                                               _lib.ptr(core.bias_pool_), _lib.ptr(core.level_scales_), _lib.ptr(tp),
                                               _lib.ptr(ta), 1, _lib.ptr(rows), _lib.cur_stream()))
     assert np.array_equal(rows.cpu().numpy(), ref_idx)
-    out = core.AnchoredQuery(tp, ta)
-    assert np.array_equal(out.detach().cpu().numpy(), ref_out)
     # int32 anchors + fp16 output + device-side count
     out16 = torch.zeros((n, 32), dtype=torch.float16, device="cuda")
     n_dev = torch.tensor([n - 7], dtype=torch.int32, device="cuda")
-    core.launch_forward(tp, ta.to(torch.int32), out_f16=out16, d_n_ptr=n_dev)
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        out = core.AnchoredQuery(tp, ta)
+        core.launch_forward(tp, ta.to(torch.int32), out_f16=out16, d_n_ptr=n_dev)
+        torch.cuda.synchronize()
+    assert fwd_prefetch_args(prof) == {"false" if log2T == 23 else "true"}
+    assert np.array_equal(out.detach().cpu().numpy(), ref_out)
     got = out16.float().cpu().numpy()
     assert np.array_equal(got[: n - 7], ref_out[: n - 7])
     assert not got[n - 7:].any()

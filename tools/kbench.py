@@ -56,7 +56,7 @@ def main():
         g16 = (torch.randn((n, 32), device="cuda") * 1e-2).half()
         gt = torch.zeros_like(core.feat_pool_)
         t = timeit(lambda: core.launch_backward(pts, anc, g16, True, gt))
-        print(f"hash bwd  [{label}] agg={os.environ.get('GF_HASH_AGG', '1')}: {t:.3f} ms  {n/t/1e6:.2f} Gpts/s  "
+        print(f"hash bwd  [{label}]: {t:.3f} ms  {n/t/1e6:.2f} Gpts/s  "
               f"{660*n/t/1e6:.0f} GB/s algorithmic")
     t = timeit(lambda: core.shadow(force=True))
     print(f"cast table: {t:.3f} ms")
