@@ -77,10 +77,8 @@ EXPORTS = ["gf_last_error", "gf_version", "gf_launch_count", "gf_mlp_param_count
 
 
 def lib():
-    global _lib, LIB_PATH
+    global _lib
     if _lib is None:
-        # development only (tools/mlp_variants.py A/B builds): another build of the SAME library
-        LIB_PATH = os.environ.get("GF_LIB_OVERRIDE", LIB_PATH)
         if not os.path.exists(LIB_PATH):
             raise RuntimeError(
                 f"{LIB_PATH} is missing: build it with `python gf-nerf_b200/build.py` "

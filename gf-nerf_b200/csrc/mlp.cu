@@ -2,7 +2,8 @@
 //
 // The per-sample layers -- the two MLPNetwork stacks of the reference field (gfnerf/mlp.py:25-57, built at
 // gfnerf/nerfacto_field.py:174-179, 217-227), trunc_exp(x + 1) (:499), the sigmoid head and their backward -- run
-// on the tcgen05 / TMEM tensor-core kernels of mlp_tc.cu.  This file holds what is constant along a ray:
+// on the tcgen05 / TMEM tensor-core kernels of mlp_tc.cu (H = 64) and mlp_tc128.cu (H = 128), which share
+// mlp_tc_common.cuh with this file (the parameter blob layout, Blob<H>).  This file holds what is constant along a ray:
 //
 //  * the head's first layer is split: SH(dir) (tcnn SH degree 4, :152-158, 521) and the appearance embedding
 //    (:530-537) are the same for every sample of a ray, so  W2[:, SH|emb] . [SH; emb] + b2  is evaluated once per
@@ -15,17 +16,9 @@
 // bench workload; the tcgen05 kernels that replaced them run 0.37 ms / 1.63 ms -- profiles/.)
 #include <stdlib.h>
 
-#include "common.cuh"
+#include "mlp_tc_common.cuh"
 
 namespace gf {
-
-// parameter blob offsets (torch nn.Linear layout), see include/gfnerf_b200.h
-template <int H>
-struct Blob {
-  static constexpr int kW0 = 0, kB0 = kW0 + H * 32, kW1 = kB0 + H, kB1 = kW1 + 16 * H, kW2 = kB1 + 16,
-                       kB2 = kW2 + H * 63, kW3 = kB2 + H, kB3 = kW3 + H * H, kW4 = kB3 + H, kB4 = kW4 + 3 * H,
-                       kParamCount = kB4 + 3;
-};
 
 // ---------------------------------------------------------------------------------------------
 // per-ray part of the head's first layer
