@@ -70,7 +70,10 @@ _SIGS = {
     "gf_peer_reduce_adam": [_int, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _vp, _f32, _vp, _vp],
     "gf_adam_step_counted": [_i64, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _vp, _f32, _int, _vp, _vp],
     "gf_adam_step": [_i64, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _i64, _f32, _int, _vp],
+    "gf_image_metrics": [_i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
+    "gf_image_metrics_scratch_bytes": [_i64, _i64, _i64],
 }
+_RET_I64 = ("gf_mlp_param_count", "gf_octree_proc_device_scratch_bytes", "gf_image_metrics_scratch_bytes")
 
 EXPORTS = ["gf_last_error", "gf_version", "gf_launch_count", "gf_mlp_param_count", "gf_mlp_mask_words",
            "gf_octree_proc_device_scratch_bytes"] + sorted(_SIGS)
@@ -95,7 +98,7 @@ def lib():
                 raise RuntimeError(f"{LIB_PATH} does not export {name}; rebuild with "
                                    "`python gf-nerf_b200/build.py --force`") from e
             fn.argtypes = sig
-            fn.restype = C.c_int64 if name in ("gf_mlp_param_count", "gf_octree_proc_device_scratch_bytes") else _int
+            fn.restype = C.c_int64 if name in _RET_I64 else _int
         _lib = L
     return _lib
 

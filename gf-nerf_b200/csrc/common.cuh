@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -52,6 +53,18 @@ inline int stride_grid(int64_t n, int block, int ctas_per_sm, int waves = 1) {
   int64_t need = div_up(n > 0 ? n : 1, block);
   int64_t cap = (int64_t)sm_count() * ctas_per_sm * waves;
   return (int)(need < cap ? need : cap);
+}
+
+// Host: the normalised fp32 Gaussian window of S3IM and SSIM, g[x] = exp(-(x - ksize/2)^2 / (2 sigma^2)) / sum, x in
+// [0, ksize); the 2-D window is the outer product g[y] * g[x].  The exponent is evaluated in double and rounded once,
+// the sum and the division in fp32.
+inline void gaussian_window(int ksize, double sigma, float* g) {
+  float gs = 0.f;
+  for (int x = 0; x < ksize; x++) {
+    g[x] = (float)exp(-(double)((x - ksize / 2) * (x - ksize / 2)) / (2.0 * sigma * sigma));
+    gs += g[x];
+  }
+  for (int x = 0; x < ksize; x++) g[x] /= gs;
 }
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }

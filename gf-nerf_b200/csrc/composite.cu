@@ -287,12 +287,8 @@ int gf_s3im(int64_t n_rays, int64_t n_virtual, const int64_t* index, const float
   GF_REQUIRE(oh > 0 && ow > 0, "gf_s3im: the window does not fit the virtual image");
   // the reference's window: fp32 Gaussian, sigma 1.5, normalised, outer product (losses.py:726-734)
   S3imWindow win;
-  float g1[8], gs = 0.f;
-  for (int x = 0; x < ksize; x++) {
-    g1[x] = (float)exp(-(double)((x - ksize / 2) * (x - ksize / 2)) / (2.0 * 1.5 * 1.5));
-    gs += g1[x];
-  }
-  for (int x = 0; x < ksize; x++) g1[x] /= gs;
+  float g1[8];
+  gaussian_window(ksize, 1.5, g1);
   for (int y = 0; y < ksize; y++)
     for (int x = 0; x < ksize; x++) win.w[y * ksize + x] = g1[y] * g1[x];
   const int64_t n_map = 3 * oh * ow;

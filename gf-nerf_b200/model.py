@@ -3,12 +3,13 @@ field -> get_weights_f2nerf -> RGB / depth / accumulation renderers -> octree fe
 `[R,1024,...]` tensors.  This is the drop-in path for callers that keep nerfstudio's Trainer / autograd / optimizers;
 `engine.GFNeRFEngine` is the same computation fused end to end on the compact layout (what bench.py times).
 """
-from typing import Dict
+from typing import Dict, Tuple
 
 import torch
 from torch import nn
 
 from .field import FieldHeadNames, GFNeRFField
+from .metrics import image_metrics
 from .perssampler import PersSampler
 from .rays import RayBundle
 from .renderers import AccumulationRenderer, DepthRenderer, RGBRenderer
@@ -47,3 +48,20 @@ class GFNeRFModel(nn.Module):
         return outputs
 
     forward = get_outputs
+
+    def get_image_metrics_and_images(self, outputs: Dict[str, torch.Tensor],
+                                     batch: Dict[str, torch.Tensor]) -> Tuple[Dict[str, float], Dict[str, torch.Tensor]]:
+        """nerfstudio's `get_image_metrics_and_images` (nerfstudio/models/nerfacto.py) on `gf_image_metrics`:
+        outputs["rgb"] and batch["image"] are one view [H, W, 3] (RGB; batch["image"] is moved to the rendered
+        image's device).  Returns metrics_dict = {"psnr": float, "ssim": float} and images_dict = {"img": ground truth
+        and rendering side by side, [H, 2W, 3]}.
+
+        LPIPS is not computed: its network weights are not part of this package, so the "lpips" key is absent -- a
+        caller that needs it keeps the reference's own method.  The accumulation and depth panels of nerfstudio's
+        images_dict are not produced either."""
+        rgb = outputs["rgb"]
+        gt = batch["image"].to(rgb.device)
+        m = image_metrics(rgb, gt)
+        metrics_dict = {"psnr": float(m["psnr"].item()), "ssim": float(m["ssim"].item())}
+        images_dict = {"img": torch.cat([gt, rgb], dim=1)}
+        return metrics_dict, images_dict

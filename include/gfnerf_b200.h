@@ -374,6 +374,27 @@ int gf_charbonnier(int64_t n_rays, const float* rgb, const float* target, float 
 int gf_s3im(int64_t n_rays, int64_t n_virtual, const int64_t* index, const float* src, const float* target,
             int patch_h, int ksize, int stride, float mult, float* g_src, float* d_loss, void* stream);
 
+/* ---- image-quality metrics of a rendered view (csrc/metrics.cu) -----------------------------------------------
+ * nerfstudio's Model.get_image_metrics_and_images for nerfacto (nerfstudio/models/nerfacto.py): torchmetrics'
+ * PeakSignalNoiseRatio(data_range=1.0) and functional structural_similarity_index_measure with its defaults, one
+ * call per image.  pred, gt: float [n_images, height, width, 3], contiguous, interleaved RGB, rows in the pixel
+ * order of the render loop (row-major), both 16-byte aligned.  Outputs float [n_images] each:
+ *   mse[b]  = sum (p - g)^2 / (3 H W), summed in double;
+ *   psnr[b] = 10 log10(1 / mse[b]); +inf when mse is 0;
+ *   ssim[b] = mean over the 3 (H - 10) (W - 10) (channel, y, x) whose 11 x 11 window lies inside the image (the
+ *             region torchmetrics keeps after its reflect pad and crop) of
+ *             ((2 mu_p mu_g + C1)(2 s_pg + C2)) / ((mu_p^2 + mu_g^2 + C1)(s_p^2 + s_g^2 + C2)),
+ *             window = outer product of the normalised Gaussian of size 11, sigma 1.5; C1 = (0.01 L)^2,
+ *             C2 = (0.03 L)^2 with L = max(max p - min p, max g - min g) over image b.  Two constant images give
+ *             L = 0 and NaN, as the formula does.
+ * scratch: gf_image_metrics_scratch_bytes(n_images, height, width) bytes, 16-byte aligned (-1: sizes invalid).
+ * Requires n_images >= 1 and height, width >= 11.  No host sync and no allocation: the call can be captured in a
+ * CUDA graph.  The work partition depends only on the sizes, so the results are bit-identical from run to run and the
+ * same for an image alone or inside a batch. */
+int64_t gf_image_metrics_scratch_bytes(int64_t n_images, int64_t height, int64_t width);
+int gf_image_metrics(int64_t n_images, int64_t height, int64_t width, const float* pred, const float* gt,
+                     float* psnr, float* ssim, float* mse, void* scratch, int64_t scratch_bytes, void* stream);
+
 /* torch.optim.Adam (no amsgrad, no weight decay) as configured at
  * gfnerf/config.py:132-135 / Hash3DAnchored.cpp:146-150.  step >= 1.
  * If shadow_f16 != NULL it is refreshed with the updated parameters.
