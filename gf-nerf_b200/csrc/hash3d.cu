@@ -16,7 +16,8 @@
 //  * backward: lanes that fall into the same grid cell (contiguous runs along the
 //    ray) are summed first -- by a 1-2 step segmented shuffle reduction for short
 //    runs, through shared memory for long ones -- and the run issues its 8
-//    vectorised fp32 reductions (red.global.add.v2.f32) once (hash_common.cuh).
+//    vectorised fp32 reductions (red.global.add.v2.f32) once (hash_common.cuh);
+//    a level whose 32 quantised gradients are all zero is left after one vote.
 //
 // Arithmetic follows the oracle's FMA convention exactly (oracle/gf_oracle.c).
 #include "common.cuh"
@@ -179,6 +180,8 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
       z = __ldg(pts + 3 * i + 2);
       vol = (int)anchors[i];
     }
+    const int pvol = __shfl_up_sync(0xffffffffu, vol, 1);  // by all 32 lanes: not inside the || below
+    const bool vol_head = lane == 0 || pvol != vol;
     if (GRAD_F16) {
       __syncwarp();  // the previous batch's readers are done with sg
       const uint4* src = reinterpret_cast<const uint4*>(grad_in_v) + base * (GF_N_LEVELS / 4);
@@ -206,7 +209,7 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
           gh = __floats2half2_rn(__fmul_rn(v.x, GF_GRAD_SCALE), __fmul_rn(v.y, GF_GRAD_SCALE));
         }
       }
-      hash_scatter_level<POW2, HAS_BIAS, UNSCALE>(l, x, y, z, vol, valid, gh, lane, n_volumes, local_size, prim_pool,
+      hash_scatter_level<POW2, HAS_BIAS, UNSCALE>(l, x, y, z, vol, vol_head, gh, lane, n_volumes, local_size, prim_pool,
                                                   bias_pool, s_scale[l], grad_table,
                                                   s_stage + (threadIdx.x >> 5) * kScatterWarpWords);
     }

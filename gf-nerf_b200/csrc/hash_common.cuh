@@ -86,45 +86,24 @@ constexpr int kScatterWarpWords = 32 * kScatterRowWords;
 // longest run of lanes the segmented shuffle reduction takes; longer runs go through shared memory
 constexpr int kScatterShuffleMaxRun = 4;
 
-// red.global.add.v2.f32 of (s0, s1) * out_scale to tab[row] unless both are zero or `mask` (0 / ~0) is off: one
-// predicated instruction, no branch and no reconvergence bookkeeping around the 8 corner updates of a level
+// `keep` of a lane that issues reductions: a sum of +0 / -0 is skipped, it would not change the table
+constexpr uint32_t kScatterKeep = 0x7fffffffu;
+
+// red.global.add.v2.f32 of (s0, s1) (times 1 / GF_GRAD_SCALE when UNSCALE) to tab[row] unless (s0 | s1) & keep is
+// zero; keep is kScatterKeep or 0 (a lane that writes nothing).  ptxas branches around a predicated reduction
+// whatever the source form, so the cost per corner is one LOP3 for the predicate, one IMAD.WIDE for the address and
+// the branch; the row is a 32-bit index into the level's 64-bit base.
 template <bool UNSCALE>
-__device__ __forceinline__ void red_add_f32x2(const char* tab, uint32_t row, float s0, float s1, uint32_t mask) {
-  constexpr float out_scale = 1.f / GF_GRAD_SCALE;
-  if (!UNSCALE) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        ".reg .b32 t;\n"
-        ".reg .b64 a;\n"
-        "or.b32 t, %2, %3;\n"
-        "and.b32 t, t, %4;\n"
-        "and.b32 t, t, 0x7fffffff;\n"
-        "setp.ne.b32 p, t, 0;\n"
-        "mad.wide.u32 a, %1, 8, %0;\n"
-        "@p red.global.add.v2.f32 [a], {%2, %3};\n"
-        "}\n" ::"l"(tab),
-        "r"(row), "f"(s0), "f"(s1), "r"(mask)
-        : "memory");
-    return;
+__device__ __forceinline__ void red_add_f32x2(float2* tab, uint32_t row, float s0, float s1, uint32_t keep) {
+  if ((__float_as_uint(s0) | __float_as_uint(s1)) & keep) {
+    constexpr float out_scale = 1.f / GF_GRAD_SCALE;
+    if (UNSCALE) {
+      s0 = __fmul_rn(s0, out_scale);
+      s1 = __fmul_rn(s1, out_scale);
+    }
+    // not atomicAdd: its unused result can still compile to an ATOM that returns the old value
+    asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(tab + row), "f"(s0), "f"(s1) : "memory");
   }
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      ".reg .b32 t;\n"
-      ".reg .b64 a;\n"
-      ".reg .f32 u, v;\n"
-      "or.b32 t, %2, %3;\n"
-      "and.b32 t, t, %4;\n"
-      "and.b32 t, t, 0x7fffffff;\n"
-      "setp.ne.b32 p, t, 0;\n"
-      "mad.wide.u32 a, %1, 8, %0;\n"
-      "mul.rn.f32 u, %2, %5;\n"
-      "mul.rn.f32 v, %3, %5;\n"
-      "@p red.global.add.v2.f32 [a], {u, v};\n"
-      "}\n" ::"l"(tab),
-      "r"(row), "f"(s0), "f"(s1), "r"(mask), "f"(out_scale)
-      : "memory");
 }
 
 // One level of the backward scatter for the 32 consecutive samples held by a warp (:81-155): recompute cell / corner
@@ -136,15 +115,18 @@ __device__ __forceinline__ void red_add_f32x2(const char* tab, uint32_t row, flo
 //   > 4      the contributions and rows go through shared memory and lane (corner d = lane & 7, quarter q = lane >> 3)
 //            walks the 8 rows of its quarter in lane order, flushing its fp32 partial sum at every run boundary:
 //            8 loads + 16 adds per lane whatever the run structure (a 5-step shuffle tree costs 80 + 80).
-// gh: this sample's two gradients of the level as fp16(g * 128).  Must be called by all 32 lanes.
+// gh: this sample's two gradients of the level as fp16(g * 128).  vol_head: lane 0, or the previous lane's sample is
+// in another volume (the same at every level, so the caller shuffles it once).  Must be called by all 32 lanes.
 // UNSCALE: the sums are divided by GF_GRAD_SCALE (:238); false leaves the table at the x128 scale for a caller that
 // folds the division into its optimizer step (exact either way: a power of two).
 template <bool POW2, bool HAS_BIAS, bool UNSCALE>
-__device__ __forceinline__ void hash_scatter_level(int l, float x, float y, float z, int vol, bool valid, __half2 gh,
+__device__ __forceinline__ void hash_scatter_level(int l, float x, float y, float z, int vol, bool vol_head, __half2 gh,
                                                    int lane, int32_t n_volumes, uint32_t local_size,
                                                    const int32_t* __restrict__ prim_pool,
                                                    const float* __restrict__ bias_pool, float scale,
                                                    float* __restrict__ grad_table, float* __restrict__ s_warp) {
+  // every product of a zero gradient is zero and no reduction of this level would be issued
+  if (!__any_sync(0xffffffffu, *reinterpret_cast<const uint32_t*>(&gh) & 0x7fff7fffu)) return;
   const int tr = (l * n_volumes + vol) * 3;
   const Cell c = cell_of(x, y, z, scale, HAS_BIAS ? bias_pool + tr : nullptr);
   const uint32_t pa = (uint32_t)__ldg(prim_pool + tr), pb = (uint32_t)__ldg(prim_pool + tr + 1),
@@ -161,11 +143,13 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
     const __half2 h = __floats2half2_rn(__fmul_rn(g0, w[d]), __fmul_rn(g1, w[d]));
     cq[d] = *reinterpret_cast<const uint32_t*>(&h);
   }
-  const char* tab = reinterpret_cast<const char*>(grad_table) + (uint64_t)level_base_row(l, local_size) * 8u;
+  // the level's first row as one 64-bit register: the opaque move keeps nvcc from folding the 64-bit base row into
+  // every corner's address (4 instructions per reduction instead of one IMAD.WIDE.U32 of the 32-bit row)
+  float2* tab = reinterpret_cast<float2*>(grad_table) + level_base_row(l, local_size);
+  asm("mov.b64 %0, %0;" : "+l"(tab));
   const uint32_t ppx = __shfl_up_sync(0xffffffffu, c.px, 1), ppy = __shfl_up_sync(0xffffffffu, c.py, 1),
                  ppz = __shfl_up_sync(0xffffffffu, c.pz, 1);
-  const int pvol = __shfl_up_sync(0xffffffffu, vol, 1);
-  const bool head = lane == 0 || ppx != c.px || ppy != c.py || ppz != c.pz || pvol != vol;
+  const bool head = vol_head || ppx != c.px || ppy != c.py || ppz != c.pz;
   const uint32_t heads = __ballot_sync(0xffffffffu, head);
   const uint32_t above = lane == 31 ? 0u : (heads & (0xffffffffu << (lane + 1)));
   const int end = above ? (__ffs(above) - 1) : 32;
@@ -176,18 +160,19 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
     for (int d = 0; d < 8; d++) row[d] = make_uint2(cq[d], pos[d]);
     __syncwarp();
     const int d = lane & 7, j0 = lane & 24;
-    const uint32_t stops = (heads >> 1) | 0x80808080u;  // bit j: lane j is the last of its run or of its quarter
-    float a0 = 0.f, a1 = 0.f;
+    // bit k: lane j0 + k is the last of its run or of its quarter
+    const uint32_t stops = ((heads >> 1) | 0x80808080u) >> j0;
+    float a0, a1;
 #pragma unroll
     for (int k = 0; k < 8; k++) {
       const uint2 e = reinterpret_cast<const uint2*>(s_warp + (j0 + k) * kScatterRowWords)[d];
       const float2 v = __half22float2(*reinterpret_cast<const __half2*>(&e.x));
-      a0 += v.x;
-      a1 += v.y;
-      if ((stops >> (j0 + k)) & 1u) {
-        red_add_f32x2<UNSCALE>(tab, e.y, a0, a1, 0xffffffffu);
-        a0 = a1 = 0.f;
-      }
+      a0 = k == 0 ? v.x : a0 + v.x;  // (not 0 + v: a -0 differs only in a zero sum, which is never written)
+      a1 = k == 0 ? v.y : a1 + v.y;
+      const bool stop = (stops >> k) & 1u;
+      red_add_f32x2<UNSCALE>(tab, e.y, a0, a1, stop ? kScatterKeep : 0u);
+      a0 = stop ? 0.f : a0;
+      a1 = stop ? 0.f : a1;
     }
     __syncwarp();  // the rows are rewritten by the next level
     return;
@@ -199,9 +184,11 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
     c0[d] = v.x;
     c1[d] = v.y;
   }
-  uint32_t writer = 0xffffffffu;  // contributions of dead lanes are already zero
+  uint32_t keep = kScatterKeep;  // contributions of dead lanes are already zero
   if (maxrun > 1) {
-    for (int off = 1; off < maxrun; off <<= 1) {
+    // two steps with fixed offsets: no loop whose trip count ptxas cannot prove uniform
+    static_assert(kScatterShuffleMaxRun == 4, "offsets 1 and 2 cover runs of up to 4 lanes");
+    auto step = [&](int off) {
       const bool take = lane + off < end;
 #pragma unroll
       for (int d = 0; d < 8; d++) {
@@ -212,11 +199,13 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
           c1[d] += o1;
         }
       }
-    }
-    writer = 0u - ((heads >> lane) & 1u);
+    };
+    step(1);
+    if (maxrun > 2) step(2);
+    keep = (heads >> lane) & 1u ? kScatterKeep : 0u;
   }
 #pragma unroll
-  for (int d = 0; d < 8; d++) red_add_f32x2<UNSCALE>(tab, pos[d], c0[d], c1[d], writer);
+  for (int d = 0; d < 8; d++) red_add_f32x2<UNSCALE>(tab, pos[d], c0[d], c1[d], keep);
 }
 
 }  // namespace gf
