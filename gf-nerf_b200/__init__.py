@@ -8,7 +8,7 @@ from .hash_3d_anchored import Hash3DAnchored, Hash3DAnchoredCore  # noqa: F401
 from .perssampler import PersSampler, PersSamplerCore  # noqa: F401
 from .engine import GFNeRFEngine  # noqa: F401
 from .field import FieldHeadNames, GFNeRFField  # noqa: F401
-from .metrics import image_metrics  # noqa: F401
+from .metrics import evaluate_views, image_metrics  # noqa: F401
 from .mlp import MLPNetwork  # noqa: F401
 from .model import GFNeRFModel  # noqa: F401
 from .cameras import Cameras  # noqa: F401

@@ -96,7 +96,203 @@ class StepOutputs:
     n_samples: torch.Tensor      # int32 [1] (device)
 
 
-class GFNeRFEngine:
+class FusedRenderer:
+    """The forward-only render body on the fused kernels -- compact sampling with the next chunk sampled ahead, hash
+    encode (+ the focal stage's residual table), ray bias, MLP, composite, the eval clamp -- over one parameter
+    source: `sampler`, `enc` (Hash3DAnchoredCore), `res` (residual Hash3DAnchoredCore or None), `mlp` (the flat MLP
+    blob, with room for a 16-byte vector tail past its end) and `emb` (appearance embedding [n_images, 32] or None).
+    `GFNeRFEngine` renders its own parameters through it; `GFNeRFModel.get_outputs_for_camera_ray_bundle` points a
+    renderer of its own at the modules' parameters (model.py)."""
+
+    def __init__(self, sampler: PersSamplerCore, hidden: int = HIDDEN):
+        self.sampler = sampler
+        self.device = sampler.device
+        self.hidden = hidden
+        self.mask_words = int(_lib.lib().gf_mlp_mask_words(hidden))
+        if self.mask_words < 0:
+            raise ValueError(f"gfnerf_b200: hidden width {hidden} is not built (64 and 128 are)")
+        self.enc = self.res = self.mlp = self.emb = None
+        self._ws = {}
+
+    # GF_NVTX=1: every stage of the step is an NVTX range ("gf/<stage>", SURVEY 8d) -- what `ncu --nvtx --nvtx-include
+    # "gf/hash_fwd/"` / an nsys timeline filter on.  Off by default: two extra host calls per stage.
+    NVTX = os.environ.get("GF_NVTX", "0") == "1"
+
+    @contextlib.contextmanager
+    def _stage(self, name):
+        ev = getattr(self, "_events", None)
+        if ev is None and not self.NVTX:
+            yield
+            return
+        if self.NVTX:
+            torch.cuda.nvtx.range_push("gf/" + name)
+        if ev is not None:
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+        try:
+            yield
+        finally:
+            if ev is not None:
+                e1.record()
+                ev.append((name, e0, e1))
+            if self.NVTX:
+                torch.cuda.nvtx.range_pop()
+
+
+    def _buf(self, name, shape, dtype, zero=False):
+        n = int(np.prod(shape))
+        t = self._ws.get(name)
+        if t is None or t.numel() < n or t.dtype != dtype:
+            t = torch.empty(max(n, 1), dtype=dtype, device=self.device)
+            self._ws[name] = t
+        t = t[:n].view(*shape)
+        if zero:
+            t.zero_()
+        return t
+
+    # ---- forward pieces --------------------------------------------------------------------
+    def _field_forward(self, cs: CompactSamples, ray_emb, train: bool = False):
+        """train: also keep the forward's ReLU masks (`relu_masks` workspace) for gf_mlp_backward"""
+        L, st = _lib.lib(), _lib.cur_stream()
+        cap, R = cs.pts01.shape[0], cs.n_rays
+        feat = self._buf("feat", (cap, 32), torch.float16)
+        sigma = self._buf("sigma", (cap,), torch.float32)
+        rgb = self._buf("rgb", (cap, 3), torch.float32)
+        ray_bias = self._buf("ray_bias", (R, self.hidden), torch.float32)
+        masks = self._buf("relu_masks", (cap, self.mask_words), torch.int32) if train else None
+        with self._stage("hash_fwd"):
+            self.enc.launch_forward(cs.pts01, cs.anchor, out_f16=feat, d_n_ptr=cs.total, recast=False)
+            if self.res is not None:
+                self.res.launch_forward_residual(cs.pts01, cs.anchor, feat, d_n_ptr=cs.total, recast=False)
+        with self._stage("ray_bias"):
+            _lib.check(L.gf_mlp_ray_bias(R, self.hidden, _lib.ptr(self.mlp), _lib.ptr(cs.rays_d),
+                                         _lib.ptr(ray_emb), _lib.ptr(ray_bias), st), "gf_mlp_ray_bias")
+        with self._stage("mlp_fwd"):
+            _lib.check(L.gf_mlp_forward(cap, _lib.ptr(cs.total), self.hidden, _lib.ptr(self.mlp), _lib.ptr(feat),
+                                        _lib.ptr(cs.ray_id), _lib.ptr(ray_bias), _lib.ptr(sigma), _lib.ptr(rgb),
+                                        _lib.ptr(masks), st), "gf_mlp_forward")
+        return feat, sigma, rgb, ray_bias
+
+    def _composite(self, cs: CompactSamples, sigma, rgb, keep: bool):
+        L, st = _lib.lib(), _lib.cur_stream()
+        cap, R = cs.pts01.shape[0], cs.n_rays
+        weights = self._buf("weights", (cap,), torch.float32) if keep else None
+        alphas = self._buf("alphas", (cap,), torch.float32) if keep else None
+        trans = self._buf("trans", (cap,), torch.float32) if keep else None
+        out_rgb = torch.empty((R, 3), dtype=torch.float32, device=self.device)
+        depth = torch.empty(R, dtype=torch.float32, device=self.device)
+        acc = torch.empty(R, dtype=torch.float32, device=self.device)
+        tmax = torch.zeros(1, dtype=torch.float32, device=self.device)
+        with self._stage("composite_fwd"):
+            _lib.check(L.gf_composite_forward(R, _lib.ptr(cs.offsets), _lib.ptr(sigma), _lib.ptr(cs.delta),
+                                              _lib.ptr(rgb), _lib.ptr(cs.t), _lib.ptr(weights), _lib.ptr(alphas),
+                                              _lib.ptr(trans), _lib.ptr(out_rgb), _lib.ptr(depth), _lib.ptr(acc),
+                                              _lib.ptr(tmax), st), "gf_composite_forward")
+        # DepthRenderer clips to the global [t.min(), t.max()] of the DENSE tensor, whose min is the padding's 0
+        # (nerfstudio/model_components/renderers.py:281)
+        depth = torch.minimum(torch.clamp_min(depth, 0.0), tmax)
+        return out_rgb, depth, acc, weights, alphas, trans
+
+    def _ray_emb(self, rel_camera_indices):
+        if self.emb is None or rel_camera_indices is None:
+            return None
+        return self.emb.index_select(0, rel_camera_indices.to(torch.int64)).contiguous()
+
+    # ---- public API ------------------------------------------------------------------------
+    @torch.no_grad()
+    def render(self, rays_o, rays_d, rel_camera_indices=None, noise=None, next_rays=None) -> StepOutputs:
+        """Forward-only (eval) pass: GFNeRFModel.get_outputs without the training feedback.  next_rays: the rays of
+        the next call, sampled on the side stream underneath this call's encode / MLP / composite (`_presample`;
+        nothing changes the octree in between)."""
+        return self._render(rays_o, rays_d, rel_camera_indices, noise, next_rays)[0]
+
+    def _render(self, rays_o, rays_d, rel_camera_indices=None, noise=None, next_rays=None):
+        """`render`, also returning the chunk's CompactSamples (valid until the sampler reuses its slot)"""
+        with torch.cuda.device(self.device):
+            cs = self._take_presampled(rays_o, rays_d) if noise is None else None
+            if cs is None:
+                cs = self.sampler.sample_compact(rays_o, rays_d, noise=noise, slot=getattr(self, "_cs_slot", 0))
+            self.flush()
+            if next_rays is not None:
+                self._presample(next_rays[0], next_rays[1])
+            _, sigma, rgb, _ = self._field_forward(cs, self._ray_emb(rel_camera_indices))
+            out_rgb, depth, acc, _, _, _ = self._composite(cs, sigma, rgb, keep=False)
+            # RGBRenderer in eval mode: nan_to_num + clamp (renderers.py:131-137)
+            out_rgb = torch.nan_to_num(out_rgb).clamp_(0.0, 1.0)
+        return StepOutputs(out_rgb, depth, acc, None, cs.total), cs
+
+    @torch.no_grad()
+    def render_rays(self, rays_o, rays_d, ray_cam=None, chunk: int = 32768, sample_ahead: bool = True,
+                    first_oct_dis: bool = False):
+        """Render of N rays in chunks of `chunk` with no host sync inside, the next chunk sampled underneath the
+        current one.  ray_cam: int64 [N], the row of `emb` each ray takes (None: no appearance embedding).  Returns
+        rgb [N,3], depth [N], acc [N] and, with `first_oct_dis`, the sampler's first_oct_dis [N] (else None)."""
+        N = rays_o.shape[0]
+        rgb = torch.empty((N, 3), dtype=torch.float32, device=self.device)
+        depth = torch.empty(N, dtype=torch.float32, device=self.device)
+        acc = torch.empty(N, dtype=torch.float32, device=self.device)
+        first = torch.empty(N, dtype=torch.float32, device=self.device) if first_oct_dis else None
+        for a in range(0, N, chunk):
+            b = min(a + chunk, N)
+            nxt = (rays_o[b:b + chunk], rays_d[b:b + chunk]) if (b < N and sample_ahead) else None
+            out, cs = self._render(rays_o[a:b], rays_d[a:b], None if ray_cam is None else ray_cam[a:b], next_rays=nxt)
+            rgb[a:b], depth[a:b], acc[a:b] = out.rgb, out.depth, out.accumulation
+            if first is not None:
+                # copied before the chunk after next is sampled into the same slot (that sampling waits on this stream)
+                first[a:b] = cs.first_oct_dis
+        return rgb, depth, acc, first
+
+    # ---- sampling one batch ahead ----------------------------------------------------------------------------
+    def _presample(self, rays_o, rays_d, vote=None, after=None):
+        """Launches the ray sampling of the NEXT batch on a side stream, ordered after everything issued so far on the
+        current stream (in particular this step's octree vote, the only thing the sampler depends on).  The sampler
+        is a latency-bound kernel that leaves most issue slots of an SM idle; the backward kernels of the current
+        batch run underneath it.  Results are identical to sampling at the start of the next step."""
+        if not hasattr(self, "_pre_stream"):
+            # GF_PRESAMPLE_PRIO=-1: the side stream's CTAs are scheduled ahead of the main stream's (A/B knob)
+            self._pre_stream = torch.cuda.Stream(device=self.device, priority=int(os.environ.get("GF_PRESAMPLE_PRIO", "0")))
+            self._pre = None
+            self._cs_slot = 0
+        cur = torch.cuda.current_stream(self.device)
+        slot = self._cs_slot ^ 1
+        # `after`: an event recorded where the side stream's inputs were complete (the forward).  Waiting on the
+        # whole current stream instead would also wait for whatever was launched since -- the MLP backward this work
+        # is meant to run underneath.
+        if after is not None:
+            self._pre_stream.wait_event(after)
+        else:
+            self._pre_stream.wait_stream(cur)
+        hook, self.sampler.stage_hook = getattr(self.sampler, "stage_hook", None), None   # events are per stream
+        with torch.cuda.stream(self._pre_stream):
+            if vote is not None:
+                # the octree feedback of the current batch (and, data parallel, its MAX all-reduce with the rank
+                # skew it absorbs) only gates the NEXT sampling: off the stream that runs the backward pass
+                vcs, weights, alphas, step = vote
+                self.sampler.update_oct_nodes_compact(vcs, weights, alphas, step)
+                self.sampler.UpdateRayMarch(step)
+            cs = self.sampler.sample_compact(rays_o, rays_d, slot=slot)
+            done = self._pre_stream.record_event()
+        self.sampler.stage_hook = hook
+        self._pre = (rays_o.data_ptr(), rays_d.data_ptr(), tuple(rays_o.shape), cs, done, slot)
+
+    def _take_presampled(self, rays_o, rays_d):
+        pre, self._pre = getattr(self, "_pre", None), None
+        if pre is None:
+            return None
+        torch.cuda.current_stream(self.device).wait_event(pre[4])    # also orders the workspace reuse
+        if pre[:3] != (rays_o.data_ptr(), rays_d.data_ptr(), tuple(rays_o.shape)):
+            return None                                              # another batch came: sample it now
+        self._cs_slot = pre[5]
+        return pre[3]
+
+    def flush(self):
+        """Orders the current stream after a sampling issued ahead on the side stream."""
+        pre = getattr(self, "_pre", None)
+        if pre is not None:
+            torch.cuda.current_stream(self.device).wait_event(pre[4])
+
+
+class GFNeRFEngine(FusedRenderer):
     """Global-stage model state (hash table, MLPs, appearance embedding) + the fused step."""
 
     # Levels per scatter launch / all-reduce message when world > 1.  16 = one scatter, one all-reduce after it (of the
@@ -111,12 +307,7 @@ class GFNeRFEngine:
                  seed: int = 0, dist_group=None, nan_guard: bool = True, s3im_loss_mult: float = 0.0,
                  s3im_kernel_size: int = 4, s3im_stride: int = 4, s3im_repeat_time: int = 10,
                  s3im_patch_height: int = 32):
-        self.sampler = sampler
-        self.device = sampler.device
-        self.hidden = hidden
-        self.mask_words = int(_lib.lib().gf_mlp_mask_words(hidden))
-        if self.mask_words < 0:
-            raise ValueError(f"gfnerf_b200: hidden width {hidden} is not built (64 and 128 are)")
+        super().__init__(sampler, hidden)
         self.nan_guard = bool(nan_guard)    # skip the optimizer step on a NaN gradient (trainer.py:416-426)
         # S3IM on top of the Charbonnier loss (gfnerf/nerfacto.py:186-197, 686-688); 0 = off
         self.s3im = (float(s3im_loss_mult), int(s3im_kernel_size), int(s3im_stride), int(s3im_repeat_time),
@@ -155,12 +346,10 @@ class GFNeRFEngine:
                                  + ([self.emb] if self.emb is not None else []))
             sampler.vote_reduce = self._peer_vote_max if self.peer is not None else self.sync.max_
         self.enc.shadow(force=True)
-        self._ws = {}
         self.step_count = 0
         self._deferred = None   # lr_scale of an optimizer step whose gradient reduce is still in flight
         self.stage = "init_stage"
-        self.res = None         # focal stage: this GPU's residual sub-encoder
-        self.opt_res = None
+        self.opt_res = None     # focal stage: Adam of this GPU's residual sub-encoder `res`
 
     # ---- focal (block) stage: reference gfnerf/nerfacto_field.py:458-489, gfnerf/nerfacto.py:432-488 ------------
     def start_block_stage(self, log2_table_size: int = None, lr: float = 5e-3, seed: int = 1):
@@ -324,35 +513,21 @@ class GFNeRFEngine:
         elif self.stage == "block_stage":
             self.end_block_stage()
 
+    @torch.no_grad()
+    def render_image(self, rays_o, rays_d, rel_camera_index: int = 0, chunk: int = 32768, sample_ahead: bool = True):
+        """Full-image render in chunks: Model.get_outputs_for_camera_ray_bundle (nerfstudio/models/base_model.py:
+        166-190, eval_num_rays_per_chunk = 2048 in the reference, gfnerf/config.py:109; here the chunk is as large
+        as the workspace allows and there is no host sync inside it).  Returns rgb [N,3], depth [N], acc [N]."""
+        cam = None
+        if self.emb is not None:
+            cam = torch.full((rays_o.shape[0],), int(rel_camera_index), dtype=torch.int64, device=self.device)
+        return self.render_rays(rays_o, rays_d, cam, chunk, sample_ahead)[:3]
+
     # ---- per-stage device timing (bench / profiling only) -----------------------------------
     def enable_timers(self, on: bool = True):
         """Brackets every stage with CUDA events on the launching stream; read with `stage_times()`."""
         self._events = [] if on else None
         self.sampler.stage_hook = self._stage if on else None
-
-    # GF_NVTX=1: every stage of the step is an NVTX range ("gf/<stage>", SURVEY 8d) -- what `ncu --nvtx --nvtx-include
-    # "gf/hash_fwd/"` / an nsys timeline filter on.  Off by default: two extra host calls per stage.
-    NVTX = os.environ.get("GF_NVTX", "0") == "1"
-
-    @contextlib.contextmanager
-    def _stage(self, name):
-        ev = getattr(self, "_events", None)
-        if ev is None and not self.NVTX:
-            yield
-            return
-        if self.NVTX:
-            torch.cuda.nvtx.range_push("gf/" + name)
-        if ev is not None:
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-        try:
-            yield
-        finally:
-            if ev is not None:
-                e1.record()
-                ev.append((name, e0, e1))
-            if self.NVTX:
-                torch.cuda.nvtx.range_pop()
 
     def stage_times(self, reset: bool = True):
         """-> {stage: (total ms, calls)} of everything recorded since the last reset (synchronises)."""
@@ -473,146 +648,6 @@ class GFNeRFEngine:
             allr = torch.empty(chunk * self.world, dtype=t.dtype, device=t.device)
             dist.all_gather_into_tensor(allr, mine, group=self.sync.group)
             t[:n] = allr[:n]
-
-    def _buf(self, name, shape, dtype, zero=False):
-        n = int(np.prod(shape))
-        t = self._ws.get(name)
-        if t is None or t.numel() < n or t.dtype != dtype:
-            t = torch.empty(max(n, 1), dtype=dtype, device=self.device)
-            self._ws[name] = t
-        t = t[:n].view(*shape)
-        if zero:
-            t.zero_()
-        return t
-
-    # ---- forward pieces --------------------------------------------------------------------
-    def _field_forward(self, cs: CompactSamples, ray_emb, train: bool = False):
-        """train: also keep the forward's ReLU masks (`relu_masks` workspace) for gf_mlp_backward"""
-        L, st = _lib.lib(), _lib.cur_stream()
-        cap, R = cs.pts01.shape[0], cs.n_rays
-        feat = self._buf("feat", (cap, 32), torch.float16)
-        sigma = self._buf("sigma", (cap,), torch.float32)
-        rgb = self._buf("rgb", (cap, 3), torch.float32)
-        ray_bias = self._buf("ray_bias", (R, self.hidden), torch.float32)
-        masks = self._buf("relu_masks", (cap, self.mask_words), torch.int32) if train else None
-        with self._stage("hash_fwd"):
-            self.enc.launch_forward(cs.pts01, cs.anchor, out_f16=feat, d_n_ptr=cs.total, recast=False)
-            if self.res is not None:
-                self.res.launch_forward_residual(cs.pts01, cs.anchor, feat, d_n_ptr=cs.total, recast=False)
-        with self._stage("ray_bias"):
-            _lib.check(L.gf_mlp_ray_bias(R, self.hidden, _lib.ptr(self.mlp), _lib.ptr(cs.rays_d),
-                                         _lib.ptr(ray_emb), _lib.ptr(ray_bias), st), "gf_mlp_ray_bias")
-        with self._stage("mlp_fwd"):
-            _lib.check(L.gf_mlp_forward(cap, _lib.ptr(cs.total), self.hidden, _lib.ptr(self.mlp), _lib.ptr(feat),
-                                        _lib.ptr(cs.ray_id), _lib.ptr(ray_bias), _lib.ptr(sigma), _lib.ptr(rgb),
-                                        _lib.ptr(masks), st), "gf_mlp_forward")
-        return feat, sigma, rgb, ray_bias
-
-    def _composite(self, cs: CompactSamples, sigma, rgb, keep: bool):
-        L, st = _lib.lib(), _lib.cur_stream()
-        cap, R = cs.pts01.shape[0], cs.n_rays
-        weights = self._buf("weights", (cap,), torch.float32) if keep else None
-        alphas = self._buf("alphas", (cap,), torch.float32) if keep else None
-        trans = self._buf("trans", (cap,), torch.float32) if keep else None
-        out_rgb = torch.empty((R, 3), dtype=torch.float32, device=self.device)
-        depth = torch.empty(R, dtype=torch.float32, device=self.device)
-        acc = torch.empty(R, dtype=torch.float32, device=self.device)
-        tmax = torch.zeros(1, dtype=torch.float32, device=self.device)
-        with self._stage("composite_fwd"):
-            _lib.check(L.gf_composite_forward(R, _lib.ptr(cs.offsets), _lib.ptr(sigma), _lib.ptr(cs.delta),
-                                              _lib.ptr(rgb), _lib.ptr(cs.t), _lib.ptr(weights), _lib.ptr(alphas),
-                                              _lib.ptr(trans), _lib.ptr(out_rgb), _lib.ptr(depth), _lib.ptr(acc),
-                                              _lib.ptr(tmax), st), "gf_composite_forward")
-        # DepthRenderer clips to the global [t.min(), t.max()] of the DENSE tensor, whose min is the padding's 0
-        # (nerfstudio/model_components/renderers.py:281)
-        depth = torch.minimum(torch.clamp_min(depth, 0.0), tmax)
-        return out_rgb, depth, acc, weights, alphas, trans
-
-    def _ray_emb(self, rel_camera_indices):
-        if self.emb is None or rel_camera_indices is None:
-            return None
-        return self.emb.index_select(0, rel_camera_indices.to(torch.int64)).contiguous()
-
-    # ---- public API ------------------------------------------------------------------------
-    @torch.no_grad()
-    def render(self, rays_o, rays_d, rel_camera_indices=None, noise=None, next_rays=None) -> StepOutputs:
-        """Forward-only (eval) pass: GFNeRFModel.get_outputs without the training feedback.  next_rays: the rays of
-        the next call, sampled on the side stream underneath this call's encode / MLP / composite (`_presample`;
-        nothing changes the octree in between)."""
-        with torch.cuda.device(self.device):
-            cs = self._take_presampled(rays_o, rays_d) if noise is None else None
-            if cs is None:
-                cs = self.sampler.sample_compact(rays_o, rays_d, noise=noise, slot=getattr(self, "_cs_slot", 0))
-            self.flush()
-            if next_rays is not None:
-                self._presample(next_rays[0], next_rays[1])
-            _, sigma, rgb, _ = self._field_forward(cs, self._ray_emb(rel_camera_indices))
-            out_rgb, depth, acc, _, _, _ = self._composite(cs, sigma, rgb, keep=False)
-            # RGBRenderer in eval mode: nan_to_num + clamp (renderers.py:131-137)
-            out_rgb = torch.nan_to_num(out_rgb).clamp_(0.0, 1.0)
-        return StepOutputs(out_rgb, depth, acc, None, cs.total)
-
-    @torch.no_grad()
-    def render_image(self, rays_o, rays_d, rel_camera_index: int = 0, chunk: int = 32768, sample_ahead: bool = True):
-        """Full-image render in chunks: Model.get_outputs_for_camera_ray_bundle (nerfstudio/models/base_model.py:
-        166-190, eval_num_rays_per_chunk = 2048 in the reference, gfnerf/config.py:109; here the chunk is as large
-        as the workspace allows and there is no host sync inside it).  Returns rgb [N,3], depth [N], acc [N]."""
-        N = rays_o.shape[0]
-        rgb = torch.empty((N, 3), dtype=torch.float32, device=self.device)
-        depth = torch.empty(N, dtype=torch.float32, device=self.device)
-        acc = torch.empty(N, dtype=torch.float32, device=self.device)
-        cam = None
-        if self.emb is not None:
-            cam = torch.full((chunk,), int(rel_camera_index), dtype=torch.int64, device=self.device)
-        for a in range(0, N, chunk):
-            b = min(a + chunk, N)
-            nxt = (rays_o[b:b + chunk], rays_d[b:b + chunk]) if (b < N and sample_ahead) else None
-            out = self.render(rays_o[a:b], rays_d[a:b], None if cam is None else cam[:b - a], next_rays=nxt)
-            rgb[a:b], depth[a:b], acc[a:b] = out.rgb, out.depth, out.accumulation
-        return rgb, depth, acc
-
-    # ---- sampling one batch ahead ----------------------------------------------------------------------------
-    def _presample(self, rays_o, rays_d, vote=None, after=None):
-        """Launches the ray sampling of the NEXT batch on a side stream, ordered after everything issued so far on the
-        current stream (in particular this step's octree vote, the only thing the sampler depends on).  The sampler
-        is a latency-bound kernel that leaves most issue slots of an SM idle; the backward kernels of the current
-        batch run underneath it.  Results are identical to sampling at the start of the next step."""
-        if not hasattr(self, "_pre_stream"):
-            # GF_PRESAMPLE_PRIO=-1: the side stream's CTAs are scheduled ahead of the main stream's (A/B knob)
-            self._pre_stream = torch.cuda.Stream(device=self.device, priority=int(os.environ.get("GF_PRESAMPLE_PRIO", "0")))
-            self._pre = None
-            self._cs_slot = 0
-        cur = torch.cuda.current_stream(self.device)
-        slot = self._cs_slot ^ 1
-        # `after`: an event recorded where the side stream's inputs were complete (the forward).  Waiting on the
-        # whole current stream instead would also wait for whatever was launched since -- the MLP backward this work
-        # is meant to run underneath.
-        if after is not None:
-            self._pre_stream.wait_event(after)
-        else:
-            self._pre_stream.wait_stream(cur)
-        hook, self.sampler.stage_hook = getattr(self.sampler, "stage_hook", None), None   # events are per stream
-        with torch.cuda.stream(self._pre_stream):
-            if vote is not None:
-                # the octree feedback of the current batch (and, data parallel, its MAX all-reduce with the rank
-                # skew it absorbs) only gates the NEXT sampling: off the stream that runs the backward pass
-                vcs, weights, alphas, step = vote
-                self.sampler.update_oct_nodes_compact(vcs, weights, alphas, step)
-                self.sampler.UpdateRayMarch(step)
-            cs = self.sampler.sample_compact(rays_o, rays_d, slot=slot)
-            done = self._pre_stream.record_event()
-        self.sampler.stage_hook = hook
-        self._pre = (rays_o.data_ptr(), rays_d.data_ptr(), tuple(rays_o.shape), cs, done, slot)
-
-    def _take_presampled(self, rays_o, rays_d):
-        pre, self._pre = getattr(self, "_pre", None), None
-        if pre is None:
-            return None
-        torch.cuda.current_stream(self.device).wait_event(pre[4])    # also orders the workspace reuse
-        if pre[:3] != (rays_o.data_ptr(), rays_d.data_ptr(), tuple(rays_o.shape)):
-            return None                                              # another batch came: sample it now
-        self._cs_slot = pre[5]
-        return pre[3]
 
     @torch.no_grad()
     def train_step(self, rays_o, rays_d, target_rgb, rel_camera_indices=None, noise=None, lr_scale: float = 1.0,
@@ -832,9 +867,7 @@ class GFNeRFEngine:
 
     def flush(self):
         """Completes a deferred optimizer step (call before reading parameters, checkpointing or timing)."""
-        pre = getattr(self, "_pre", None)
-        if pre is not None:   # an octree vote / sampling issued ahead on the side stream
-            torch.cuda.current_stream(self.device).wait_event(pre[4])
+        super().flush()       # an octree vote / sampling issued ahead on the side stream
         if self._deferred is not None:
             self.sync.wait()
             self._apply_adam(self._deferred)

@@ -1,8 +1,9 @@
 """Image-quality metrics of rendered views on the device: PSNR, SSIM and MSE per image in one kernel sequence
 (`gf_image_metrics`, csrc/metrics.cu).  The conventions are those of nerfstudio's nerfacto evaluation -- torchmetrics'
 `PeakSignalNoiseRatio(data_range=1.0)` and functional `structural_similarity_index_measure` with its defaults, one
-call per image; see include/gfnerf_b200.h."""
-from typing import Dict
+call per image; see include/gfnerf_b200.h.  `evaluate_views` is the held-out evaluation loop around them."""
+import time
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
 
@@ -39,3 +40,48 @@ def _aligned(t: torch.Tensor) -> torch.Tensor:
     """contiguous and 16-byte aligned (the kernels load 16-byte blocks); a view into the middle of a tensor is copied"""
     t = t.contiguous()
     return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+def evaluate_views(model, cameras, images, camera_indices: Optional[Sequence[int]] = None
+                   ) -> Tuple[Dict[str, float], List[Dict[str, float]]]:
+    """The body of nerfstudio's `Pipeline.get_average_eval_image_metrics` (nerfstudio/pipelines/base_pipeline.py)
+    without the datamanager.  `cameras`: a `Cameras` with `width` and `height` set; `images`: one ground truth per
+    evaluated camera, [H, W, 3] fp32, on the device or the host; `camera_indices`: the cameras to evaluate (default:
+    all, in order).  Per view: the frame's rays (`gf_generate_rays`) as an [H, W] bundle ->
+    `model.get_outputs_for_camera_ray_bundle` -> `model.get_image_metrics_and_images`, plus `num_rays_per_sec`
+    = H * W / wall time and `fps` = 1 / wall time, host clock from the render to the metrics' `.item()`.  The bundle
+    has no `rel_camera_indices`: the model picks the appearance embedding by its nearest-camera rule, as the
+    reference's evaluation does.  Returns (averages: the mean of every key plus `psnr_std` and `ssim_std`, the
+    unbiased std of torch.std_mean as nerfstudio reports it; per_image: one dict per view)."""
+    from .rays import RayBundle
+    idx = list(range(len(cameras))) if camera_indices is None else [int(i) for i in camera_indices]
+    if len(images) != len(idx):
+        raise RuntimeError(f"evaluate_views: {len(images)} images for {len(idx)} cameras")
+    H, W = int(cameras.height), int(cameras.width)
+    per_image = []
+    for i, gt in zip(idx, images):
+        if tuple(gt.shape) != (H, W, 3):
+            raise RuntimeError(f"evaluate_views: ground truth of camera {i} is {tuple(gt.shape)}, the camera renders "
+                               f"({H}, {W}, 3)")
+        rays = cameras.generate_frame_rays(i)
+        bundle = RayBundle(origins=rays.origins.view(H, W, 3), directions=rays.directions.view(H, W, 3),
+                           lookat_directions=rays.lookat_directions.view(H, W, 3),
+                           pixel_area=rays.pixel_area.view(H, W, 1), camera_indices=rays.camera_indices.view(H, W, 1),
+                           metadata=rays.metadata)
+        torch.cuda.synchronize(rays.origins.device)
+        t0 = time.perf_counter()
+        outputs = model.get_outputs_for_camera_ray_bundle(bundle)
+        metrics, _ = model.get_image_metrics_and_images(outputs, {"image": gt})
+        dt = time.perf_counter() - t0
+        metrics["num_rays_per_sec"] = H * W / dt
+        metrics["fps"] = 1.0 / dt
+        per_image.append(metrics)
+    averages = {}
+    for key in per_image[0] if per_image else ():
+        vals = torch.tensor([m[key] for m in per_image], dtype=torch.float64)
+        if key in ("psnr", "ssim"):
+            std, mean = torch.std_mean(vals)
+            averages[key], averages[key + "_std"] = float(mean), float(std)
+        else:
+            averages[key] = float(vals.mean())
+    return averages, per_image

@@ -2,12 +2,15 @@
 field -> get_weights_f2nerf -> RGB / depth / accumulation renderers -> octree feedback, on the reference's dense
 `[R,1024,...]` tensors.  This is the drop-in path for callers that keep nerfstudio's Trainer / autograd / optimizers;
 `engine.GFNeRFEngine` is the same computation fused end to end on the compact layout (what bench.py times).
+`get_outputs_for_camera_ray_bundle` renders whole views of the modules' parameters through that fused path.
 """
 from typing import Dict, Tuple
 
 import torch
 from torch import nn
 
+from . import _lib
+from .engine import FusedRenderer
 from .field import FieldHeadNames, GFNeRFField
 from .metrics import image_metrics
 from .perssampler import PersSampler
@@ -24,6 +27,7 @@ class GFNeRFModel(nn.Module):
         self.renderer_rgb = RGBRenderer(background_color=background_color)
         self.renderer_accumulation = AccumulationRenderer()
         self.renderer_depth = DepthRenderer(method="expected")     # gfnerf/nerfacto.py:288
+        self._fused = None        # FusedRenderer of get_outputs_for_camera_ray_bundle, made at its first call
 
     def get_outputs(self, ray_bundle: RayBundle) -> Dict[str, torch.Tensor]:
         ray_samples = self.persampler(ray_bundle)
@@ -48,6 +52,70 @@ class GFNeRFModel(nn.Module):
         return outputs
 
     forward = get_outputs
+
+    # rays per get_outputs call in the reference's evaluation (eval_num_rays_per_chunk, gfnerf/config.py:109); the
+    # appearance embedding of a view is chosen per chunk of this many rays
+    EVAL_NUM_RAYS_PER_CHUNK = 2048
+
+    @torch.no_grad()
+    def get_outputs_for_camera_ray_bundle(self, camera_ray_bundle: RayBundle, chunk: int = 32768) -> Dict[str, torch.Tensor]:
+        """nerfstudio's `Model.get_outputs_for_camera_ray_bundle` (nerfstudio/models/base_model.py:166-190) on the fused
+        kernels: `get_outputs` in eval mode over a whole view, `chunk` rays per fused render with no host sync in
+        between.  origins / directions are [H, W, 3] (any leading shape works); returns {"rgb": [H,W,3],
+        "accumulation", "depth", "oct_depth": [H,W,1]}.
+
+        The parameters are the modules' as they are at the call: the global table, the MLP blob, the appearance
+        embedding and, in the block stage, the residual table `base_encoding_{i}` of `field.active_block_idxs_test`.
+        The fp16 table copies and the MLP blob are refreshed once per call; nothing is copied into an engine and no
+        optimizer state is made.  Rays take the embedding row of `rel_camera_indices` if the bundle has them, else
+        the one of the training camera nearest to the first origin of their 2048-ray chunk, as the reference's
+        `PersSampler.generate_ray_samples` chooses it for each `get_outputs` call of its evaluation loop.  The octree
+        is not updated and `self.training` is left as it is; the march noise follows the sampler's mode."""
+        f, rb = self.field, camera_ray_bundle
+        shape = tuple(rb.origins.shape[:-1])
+        _lib.require_cuda(rb.origins, rb.directions)
+        o = rb.origins.reshape(-1, 3).contiguous().float()
+        d = rb.directions.reshape(-1, 3).contiguous().float()
+        n = o.shape[0]
+        r = self._fused
+        if r is None or r.sampler is not self.persampler.sampler or r.hidden != f.hidden_dim:
+            r = self._fused = FusedRenderer(self.persampler.sampler, f.hidden_dim)
+        r.enc, r.res = f.base_encoding_init.hash_3d, None
+        if f.cur_stage == "block_stage":
+            if len(f.active_block_idxs_test) != 1:
+                raise RuntimeError(f"get_outputs_for_camera_ray_bundle: the block stage renders one block table, "
+                                   f"active_block_idxs_test is {f.active_block_idxs_test}")
+            r.res = getattr(f, f"base_encoding_{f.active_block_idxs_test[0]}").hash_3d
+        for enc in (r.enc, r.res):
+            if enc is not None:
+                enc.shadow(force=True)
+                enc._bias()          # the all-zero test of the bias pool (a host read) before the chunk loop
+        blob = torch.cat([f.base_network.flat_params(), f.mlp_head.flat_params()]).float()
+        if r.mlp is None or r.mlp.numel() != blob.numel():
+            # the MLP kernels load a 16-byte vector tail past the blob (as for GFNeRFEngine.mlp)
+            r.mlp = torch.zeros((blob.numel() + 3) // 4 * 4, device=r.device)[:blob.numel()]
+        r.mlp.copy_(blob)
+        r.emb, cam = None, None
+        if f.use_appearance_embedding:
+            r.emb = f.embedding_appearance.embedding.weight.detach()
+            if rb.rel_camera_indices is not None:
+                cam = rb.rel_camera_indices.reshape(n, -1)[:, 0].to(device=r.device, dtype=torch.int64)
+            else:
+                cam = self._nearest_cameras(o)
+        rgb, depth, acc, first = r.render_rays(o, d, cam, chunk=chunk, first_oct_dis=True)
+        return {"rgb": rgb.view(*shape, 3), "accumulation": acc.view(*shape, 1),
+                "depth": (depth / self.scale_factor).view(*shape, 1),
+                "oct_depth": (first / self.scale_factor).view(*shape, 1)}
+
+    def _nearest_cameras(self, origins: torch.Tensor) -> torch.Tensor:
+        """int64 [N]: per ray, the training camera nearest to the first origin of its EVAL_NUM_RAYS_PER_CHUNK-ray chunk,
+        with the distance and argmin of `PersSampler.get_nearest_split_dataset*`; on the device, no host read."""
+        k = self.EVAL_NUM_RAYS_PER_CHUNK
+        c2w = self.persampler.c2w
+        firsts = origins[::k].to(c2w.device)                                        # [chunks, 3]
+        dists = torch.linalg.norm(c2w[None, :, 0:3, -1] - firsts[:, None, :], dim=2)   # [chunks, cameras]
+        nearest = torch.argmin(dists, dim=1)
+        return nearest.view(-1, 1).expand(-1, k).reshape(-1)[:origins.shape[0]].to(origins.device)
 
     def get_image_metrics_and_images(self, outputs: Dict[str, torch.Tensor],
                                      batch: Dict[str, torch.Tensor]) -> Tuple[Dict[str, float], Dict[str, torch.Tensor]]:
