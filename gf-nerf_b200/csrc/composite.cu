@@ -61,7 +61,10 @@ composite_fwd_kernel(int64_t n_rays, const int* __restrict__ offsets, const floa
         const float y = __shfl_up_sync(0xffffffffu, incl, off);
         if (lane >= off) incl += y;
       }
-      const float excl = carry + (incl - dd);
+      // exclusive prefix = the previous lane's inclusive sum: incl - dd would lose the earlier samples' sum to
+      // ulp(dd) at an opaque sample and turn it into NaN at dd = inf
+      const float prev = __shfl_up_sync(0xffffffffu, incl, 1);
+      const float excl = carry + (lane > 0 ? prev : 0.f);
       const float alpha = 1.f - expf(-dd);
       const float T = expf(-excl);
       const float w = nan_to_num(alpha * T);
@@ -144,7 +147,9 @@ composite_bwd_kernel(int64_t n_rays, const int* __restrict__ offsets, const floa
         const float y = __shfl_down_sync(0xffffffffu, incl, off);
         if (lane + off < 32) incl += y;
       }
-      const float behind = carry + (incl - own);
+      // exclusive suffix = the next lane's inclusive suffix, never incl - own (see the forward)
+      const float next = __shfl_down_sync(0xffffffffu, incl, 1);
+      const float behind = carry + (lane < 31 ? next : 0.f);
       if (valid) {
         d_sigma[s] = (gw * e * T - behind) * dl;
         if (d_rgb) {
@@ -256,6 +261,7 @@ int gf_composite_backward(int64_t n_rays, const int32_t* offsets, const float* s
   GF_REQUIRE(n_rays >= 0, "gf_composite_backward: bad sizes");
   if (n_rays == 0) return GF_OK;
   GF_REQUIRE(offsets && sigma && delta && trans && d_sigma, "gf_composite_backward: null pointer");
+  GF_REQUIRE(!g_rgb || rgb, "gf_composite_backward: g_rgb without rgb");
   GF_REQUIRE(!d_rgb || (g_rgb && rgb), "gf_composite_backward: d_rgb needs g_rgb and rgb");
   const int grid = stride_grid(n_rays * 32, kCompBlock, 8, 2);
   composite_bwd_kernel<<<grid, kCompBlock, 0, (cudaStream_t)stream>>>(n_rays, offsets, sigma, delta, rgb, trans,
@@ -283,8 +289,9 @@ int gf_s3im(int64_t n_rays, int64_t n_virtual, const int64_t* index, const float
   GF_REQUIRE(index && src && target, "gf_s3im: null pointer");
   const int64_t W = n_virtual / patch_h;
   const int pad = (ksize - 1) / 2;
+  // checked before the division, which truncates toward zero: a window one row too tall would still give oh = 1
+  GF_REQUIRE(patch_h + 2 * pad >= ksize && W + 2 * pad >= ksize, "gf_s3im: the window does not fit the virtual image");
   const int64_t oh = (patch_h + 2 * pad - ksize) / stride + 1, ow = (W + 2 * pad - ksize) / stride + 1;
-  GF_REQUIRE(oh > 0 && ow > 0, "gf_s3im: the window does not fit the virtual image");
   // the reference's window: fp32 Gaussian, sigma 1.5, normalised, outer product (losses.py:726-734)
   S3imWindow win;
   float g1[8];
