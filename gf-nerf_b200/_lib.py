@@ -27,6 +27,8 @@ _SIGS = {
     "gf_hash_cast_table": [_vp, _vp, _i64, _vp],
     "gf_hash_forward": [_i64, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp],
     "gf_hash_forward_residual": [_i64, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp],
+    "gf_hash_forward_residual_routed": [_i64, _vp, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp, _vp,
+                                        _vp],
     "gf_hash_backward": [_i64, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _int, _vp, _vp],
     "gf_hash_backward_levels": [_i64, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _int, _vp, _int, _int, _vp],
     "gf_hash_corner_rows": [_i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _vp],

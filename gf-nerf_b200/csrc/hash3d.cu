@@ -56,13 +56,43 @@ constexpr int kHashBlock = 256;
 //                     3 CTAs per SM -- best while the reachable rows fit the L2 and the kernel is bound by the L1 -> L2
 //                     request path, not by DRAM latency (log2T = 19: 0.949 ms against 0.985; log2T = 21, 71 MB of
 //                     rows: 0.970 against 1.338).
-template <bool POW2, typename AnchorT, bool OUT16, bool OUT32, bool PREFETCH>
-__global__ void __launch_bounds__(kHashBlock, PREFETCH ? 3 : 5)
-hash_fwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes, uint32_t local_size,
-                const __half2* __restrict__ feat, const int32_t* __restrict__ prim_pool,
-                const float* __restrict__ bias_pool, const float* __restrict__ scales,
-                const float* __restrict__ pts, const AnchorT* __restrict__ anchors,
-                uint4* __restrict__ out16, float4* __restrict__ out32, const uint4* __restrict__ base16) {
+// The table a sample reads.  `OneTable`: every sample the same (hash_fwd_kernel).  `RoutedTables`: sample i takes
+// table ray_table[ray_id[i]] of a device descriptor array (hash_fwd_routed_kernel); an id outside [0, n_tables)
+// selects none, and the sample's base row is passed through.
+struct OneTable {
+  const __half2* __restrict__ feat;
+  const int32_t* __restrict__ prim_pool;
+  const float* __restrict__ bias_pool;
+  __device__ __forceinline__ bool operator()(int64_t, const __half2*& f, const int32_t*& p, const float*& b) const {
+    f = feat;
+    p = prim_pool;
+    b = bias_pool;
+    return true;
+  }
+};
+
+struct RoutedTables {
+  const gf_hash_table_ref* __restrict__ tables;
+  int32_t n_tables;
+  const int32_t* __restrict__ ray_id;
+  const int32_t* __restrict__ ray_table;
+  __device__ __forceinline__ bool operator()(int64_t i, const __half2*& f, const int32_t*& p, const float*& b) const {
+    const int32_t t = __ldg(ray_table + __ldg(ray_id + i));
+    if ((uint32_t)t >= (uint32_t)n_tables) return false;
+    f = reinterpret_cast<const __half2*>(__ldg(reinterpret_cast<const unsigned long long*>(&tables[t].feat_f16)));
+    p = reinterpret_cast<const int32_t*>(__ldg(reinterpret_cast<const unsigned long long*>(&tables[t].prim_pool)));
+    b = reinterpret_cast<const float*>(__ldg(reinterpret_cast<const unsigned long long*>(&tables[t].bias_pool)));
+    return true;
+  }
+};
+
+// The forward gather of hash_fwd_kernel and hash_fwd_routed_kernel: one thread per sample, all 16 levels.
+template <bool POW2, typename AnchorT, bool OUT16, bool OUT32, bool PREFETCH, typename Tables>
+__device__ __forceinline__ void hash_fwd_body(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes,
+                                              uint32_t local_size, const Tables& table,
+                                              const float* __restrict__ scales, const float* __restrict__ pts,
+                                              const AnchorT* __restrict__ anchors, uint4* __restrict__ out16,
+                                              float4* __restrict__ out32, const uint4* __restrict__ base16) {
   if (d_n_ptr) {
     int64_t dn = *d_n_ptr;
     n = dn < n ? dn : n;
@@ -72,6 +102,16 @@ hash_fwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
   __syncthreads();
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const __half2* feat;
+    const int32_t* prim_pool;
+    const float* bias_pool;
+    if (!table(i, feat, prim_pool, bias_pool)) {   // routed, no table: the base row unchanged
+      if ((const void*)out16 != (const void*)base16) {
+#pragma unroll
+        for (int q = 0; q < GF_N_LEVELS / 4; q++) out16[i * 4 + q] = __ldg(base16 + i * 4 + q);
+      }
+      continue;
+    }
     const float x = __ldg(pts + 3 * i), y = __ldg(pts + 3 * i + 1), z = __ldg(pts + 3 * i + 2);
     const int vol = (int)anchors[i];
 #pragma unroll 1
@@ -142,6 +182,32 @@ hash_fwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
       }
     }
   }
+}
+
+template <bool POW2, typename AnchorT, bool OUT16, bool OUT32, bool PREFETCH>
+__global__ void __launch_bounds__(kHashBlock, PREFETCH ? 3 : 5)
+hash_fwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes, uint32_t local_size,
+                const __half2* __restrict__ feat, const int32_t* __restrict__ prim_pool,
+                const float* __restrict__ bias_pool, const float* __restrict__ scales,
+                const float* __restrict__ pts, const AnchorT* __restrict__ anchors,
+                uint4* __restrict__ out16, float4* __restrict__ out32, const uint4* __restrict__ base16) {
+  hash_fwd_body<POW2, AnchorT, OUT16, OUT32, PREFETCH>(n, d_n_ptr, n_volumes, local_size,
+                                                       OneTable{feat, prim_pool, bias_pool}, scales, pts, anchors,
+                                                       out16, out32, base16);
+}
+
+// Residual gather with a table per sample (gf_hash_forward_residual_routed): fp16 output on top of base16 only.
+// Same register budget and occupancy as hash_fwd_kernel's variant of the same PREFETCH.
+template <bool POW2, typename AnchorT, bool PREFETCH>
+__global__ void __launch_bounds__(kHashBlock, PREFETCH ? 3 : 5)
+hash_fwd_routed_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes, uint32_t local_size,
+                       int32_t n_tables, const gf_hash_table_ref* __restrict__ tables,
+                       const float* __restrict__ scales, const float* __restrict__ pts,
+                       const AnchorT* __restrict__ anchors, const int32_t* __restrict__ ray_id,
+                       const int32_t* __restrict__ ray_table, uint4* out16, const uint4* base16) {
+  hash_fwd_body<POW2, AnchorT, true, false, PREFETCH>(n, d_n_ptr, n_volumes, local_size,
+                                                      RoutedTables{tables, n_tables, ray_id, ray_table}, scales, pts,
+                                                      anchors, out16, nullptr, base16);
 }
 
 template <bool POW2, typename AnchorT, bool GRAD_F16, bool HAS_BIAS, bool UNSCALE>
@@ -332,6 +398,42 @@ int gf_hash_forward_residual(int64_t n, const int32_t* d_n_ptr, int32_t n_volume
   GF_REQUIRE(base_f16 && out_f16, "gf_hash_forward_residual: null base / output");
   return hash_forward_impl(n, d_n_ptr, n_volumes, local_size, feat_f16, prim_pool, bias_pool, level_scales, pts,
                            anchors, anchor_i64, out_f16, nullptr, base_f16, stream);
+}
+
+int gf_hash_forward_residual_routed(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes, int64_t local_size,
+                                    int32_t n_tables, const gf_hash_table_ref* d_tables, const float* level_scales,
+                                    const float* pts, const void* anchors, int anchor_i64, const int32_t* ray_id,
+                                    const int32_t* ray_table, const void* base_f16, void* out_f16, void* stream) {
+  GF_REQUIRE(n >= 0 && n_volumes > 0 && local_size > 0 && local_size <= 0x7fffffffLL && local_size % 2 == 0,
+             "gf_hash_forward_residual_routed: bad sizes n=%lld n_volumes=%d local_size=%lld (must be even)",
+             (long long)n, n_volumes, (long long)local_size);
+  GF_REQUIRE((int64_t)n_volumes * GF_N_LEVELS * 3 <= 0x7fffffffLL, "gf_hash_forward_residual_routed: n_volumes too large");
+  GF_REQUIRE(n_tables > 0, "gf_hash_forward_residual_routed: n_tables = %d (must be > 0)", n_tables);
+  GF_REQUIRE(d_tables && ray_id && ray_table && base_f16 && out_f16,
+             "gf_hash_forward_residual_routed: null table descriptors / ray_id / ray_table / base / output");
+  if (n == 0) return GF_OK;
+  GF_REQUIRE(level_scales && pts && anchors, "gf_hash_forward_residual_routed: null pointer");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int grid = stride_grid(n, kHashBlock, 8, 4);
+  const bool p2 = is_pow2(local_size);
+  const bool l2_resident = (int64_t)local_size * 34 <= (int64_t)100 << 20;   // as hash_forward_impl
+#define GF_FWD_R(P2, AT, PF)                                                                                    \
+  hash_fwd_routed_kernel<P2, AT, PF><<<grid, kHashBlock, 0, st>>>(                                              \
+      n, d_n_ptr, n_volumes, (uint32_t)local_size, n_tables, d_tables, level_scales, pts, (const AT*)anchors,   \
+      ray_id, ray_table, (uint4*)out_f16, (const uint4*)base_f16)
+#define GF_FWD_RA(P2, AT)                        \
+  do {                                           \
+    if (l2_resident) GF_FWD_R(P2, AT, true);     \
+    else GF_FWD_R(P2, AT, false);                \
+  } while (0)
+  if (p2) {
+    if (anchor_i64) GF_FWD_RA(true, int64_t); else GF_FWD_RA(true, int32_t);
+  } else {
+    if (anchor_i64) GF_FWD_RA(false, int64_t); else GF_FWD_RA(false, int32_t);
+  }
+#undef GF_FWD_RA
+#undef GF_FWD_R
+  return check_launch("hash_fwd_routed_kernel");
 }
 
 int gf_hash_backward(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes, int64_t local_size,

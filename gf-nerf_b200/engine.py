@@ -101,6 +101,8 @@ class FusedRenderer:
     encode (+ the focal stage's residual table), ray bias, MLP, composite, the eval clamp -- over one parameter
     source: `sampler`, `enc` (Hash3DAnchoredCore), `res` (residual Hash3DAnchoredCore or None), `mlp` (the flat MLP
     blob, with room for a 16-byte vector tail past its end) and `emb` (appearance embedding [n_images, 32] or None).
+    `res_tables` = (cores, refs) instead of `res`: several residual tables, each ray taking the one its `ray_table`
+    entry names (`Hash3DAnchoredCore.launch_forward_residual_routed`; refs from `Hash3DAnchoredCore.table_refs`).
     `GFNeRFEngine` renders its own parameters through it; `GFNeRFModel.get_outputs_for_camera_ray_bundle` points a
     renderer of its own at the modules' parameters (model.py)."""
 
@@ -111,7 +113,7 @@ class FusedRenderer:
         self.mask_words = int(_lib.lib().gf_mlp_mask_words(hidden))
         if self.mask_words < 0:
             raise ValueError(f"gfnerf_b200: hidden width {hidden} is not built (64 and 128 are)")
-        self.enc = self.res = self.mlp = self.emb = None
+        self.enc = self.res = self.mlp = self.emb = self.res_tables = None
         self._ws = {}
 
     # GF_NVTX=1: every stage of the step is an NVTX range ("gf/<stage>", SURVEY 8d) -- what `ncu --nvtx --nvtx-include
@@ -151,8 +153,9 @@ class FusedRenderer:
         return t
 
     # ---- forward pieces --------------------------------------------------------------------
-    def _field_forward(self, cs: CompactSamples, ray_emb, train: bool = False):
-        """train: also keep the forward's ReLU masks (`relu_masks` workspace) for gf_mlp_backward"""
+    def _field_forward(self, cs: CompactSamples, ray_emb, train: bool = False, ray_table=None):
+        """train: also keep the forward's ReLU masks (`relu_masks` workspace) for gf_mlp_backward.  ray_table: int32
+        [n_rays], each ray's index into `res_tables` (used only when `res_tables` is set)"""
         L, st = _lib.lib(), _lib.cur_stream()
         cap, R = cs.pts01.shape[0], cs.n_rays
         feat = self._buf("feat", (cap, 32), torch.float16)
@@ -162,7 +165,13 @@ class FusedRenderer:
         masks = self._buf("relu_masks", (cap, self.mask_words), torch.int32) if train else None
         with self._stage("hash_fwd"):
             self.enc.launch_forward(cs.pts01, cs.anchor, out_f16=feat, d_n_ptr=cs.total, recast=False)
-            if self.res is not None:
+            if self.res_tables is not None:
+                if ray_table is None:
+                    raise ValueError("gfnerf_b200: several residual tables are set, but no per-ray ray_table")
+                cores, refs = self.res_tables
+                Hash3DAnchoredCore.launch_forward_residual_routed(cores, cs.pts01, cs.anchor, feat, cs.ray_id, ray_table,
+                                                                  d_n_ptr=cs.total, refs=refs)
+            elif self.res is not None:
                 self.res.launch_forward_residual(cs.pts01, cs.anchor, feat, d_n_ptr=cs.total, recast=False)
         with self._stage("ray_bias"):
             _lib.check(L.gf_mlp_ray_bias(R, self.hidden, _lib.ptr(self.mlp), _lib.ptr(cs.rays_d),
@@ -206,7 +215,7 @@ class FusedRenderer:
         nothing changes the octree in between)."""
         return self._render(rays_o, rays_d, rel_camera_indices, noise, next_rays)[0]
 
-    def _render(self, rays_o, rays_d, rel_camera_indices=None, noise=None, next_rays=None):
+    def _render(self, rays_o, rays_d, rel_camera_indices=None, noise=None, next_rays=None, ray_table=None):
         """`render`, also returning the chunk's CompactSamples (valid until the sampler reuses its slot)"""
         with torch.cuda.device(self.device):
             cs = self._take_presampled(rays_o, rays_d) if noise is None else None
@@ -215,7 +224,7 @@ class FusedRenderer:
             self.flush()
             if next_rays is not None:
                 self._presample(next_rays[0], next_rays[1])
-            _, sigma, rgb, _ = self._field_forward(cs, self._ray_emb(rel_camera_indices))
+            _, sigma, rgb, _ = self._field_forward(cs, self._ray_emb(rel_camera_indices), ray_table=ray_table)
             out_rgb, depth, acc, _, _, _ = self._composite(cs, sigma, rgb, keep=False)
             # RGBRenderer in eval mode: nan_to_num + clamp (renderers.py:131-137)
             out_rgb = torch.nan_to_num(out_rgb).clamp_(0.0, 1.0)
@@ -223,10 +232,11 @@ class FusedRenderer:
 
     @torch.no_grad()
     def render_rays(self, rays_o, rays_d, ray_cam=None, chunk: int = 32768, sample_ahead: bool = True,
-                    first_oct_dis: bool = False):
+                    first_oct_dis: bool = False, ray_table=None):
         """Render of N rays in chunks of `chunk` with no host sync inside, the next chunk sampled underneath the
-        current one.  ray_cam: int64 [N], the row of `emb` each ray takes (None: no appearance embedding).  Returns
-        rgb [N,3], depth [N], acc [N] and, with `first_oct_dis`, the sampler's first_oct_dis [N] (else None)."""
+        current one.  ray_cam: int64 [N], the row of `emb` each ray takes (None: no appearance embedding).  ray_table:
+        int32 [N], the entry of `res_tables` each ray takes (with `res_tables` only).  Returns rgb [N,3], depth [N],
+        acc [N] and, with `first_oct_dis`, the sampler's first_oct_dis [N] (else None)."""
         N = rays_o.shape[0]
         rgb = torch.empty((N, 3), dtype=torch.float32, device=self.device)
         depth = torch.empty(N, dtype=torch.float32, device=self.device)
@@ -235,7 +245,8 @@ class FusedRenderer:
         for a in range(0, N, chunk):
             b = min(a + chunk, N)
             nxt = (rays_o[b:b + chunk], rays_d[b:b + chunk]) if (b < N and sample_ahead) else None
-            out, cs = self._render(rays_o[a:b], rays_d[a:b], None if ray_cam is None else ray_cam[a:b], next_rays=nxt)
+            out, cs = self._render(rays_o[a:b], rays_d[a:b], None if ray_cam is None else ray_cam[a:b], next_rays=nxt,
+                                   ray_table=None if ray_table is None else ray_table[a:b])
             rgb[a:b], depth[a:b], acc[a:b] = out.rgb, out.depth, out.accumulation
             if first is not None:
                 # copied before the chunk after next is sampled into the same slot (that sampling waits on this stream)
@@ -417,12 +428,21 @@ class GFNeRFEngine(FusedRenderer):
                     opt.m.zero_(), opt.v.zero_(), opt.d_step.zero_()
         self.enc.shadow(force=True)
 
-    def store_model(self, model):
+    def store_model(self, model, block: Optional[int] = None):
         """The inverse of `load_model`: the engine's current parameters into the field's modules (whose `state_dict()`
-        is the reference's checkpoint layout)."""
+        is the reference's checkpoint layout).  block = b (block stage only): the residual table `res` also goes into
+        the field's `base_encoding_{b}`, which is created if the field has none -- how the blocks of a focal run,
+        one per rank, are gathered into one model (each rank stores its block, then `field.save_table(b)`)."""
         f = getattr(model, "field", model)
         if int(f.hidden_dim) != self.hidden:
             raise ValueError(f"gfnerf_b200: the field is {f.hidden_dim} wide, the engine {self.hidden}")
+        if block is not None:
+            if self.stage != "block_stage" or self.res is None:
+                raise ValueError(f"gfnerf_b200: store_model(block={block}) needs the block stage; the engine is in "
+                                 f"{self.stage}")
+            if int(f.log2_table_size) != int(np.log2(self.res.local_size_)):
+                raise ValueError(f"gfnerf_b200: the field's block tables are 2^{f.log2_table_size} rows per level, "
+                                 f"the engine's residual table 2^{int(np.log2(self.res.local_size_))}")
         self.flush()
         self.sync_master_params()       # peer exchange: every rank only keeps ITS fp32 rows current
         f.base_encoding_init.load_states([t.detach() for t in self.enc.States()], 0)
@@ -435,6 +455,11 @@ class GFNeRFEngine(FusedRenderer):
             if self.emb is not None:
                 f.embedding_appearance.embedding.weight.copy_(self.emb)
         assert o == self.mlp.numel()
+        if block is not None:
+            name = f"base_encoding_{int(block)}"
+            if not hasattr(f, name):
+                f.add_table(int(block))
+            getattr(f, name).load_states([t.detach() for t in self.res.States()], 0)
 
     # ---- resume ---------------------------------------------------------------------------------------------------------
     def checkpoint(self) -> dict:

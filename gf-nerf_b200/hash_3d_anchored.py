@@ -177,6 +177,42 @@ class Hash3DAnchoredCore:
                 _lib.ptr(self.level_scales_), _lib.ptr(points), _lib.ptr(anchors), int(anchors.dtype == torch.int64),
                 _lib.ptr(base_f16), _lib.ptr(out_f16), _lib.cur_stream()), "gf_hash_forward_residual")
 
+    @staticmethod
+    def table_refs(cores, device, recast=True) -> torch.Tensor:
+        """The gf_hash_table_ref array of `cores` on `device` (int64 [K, 3]: fp16 shadow, prime pool, bias pool or 0),
+        for `launch_forward_residual_routed`.  The shadows are refreshed first (recast); the array holds their
+        addresses, so it is valid until one of the tables is reallocated.  The bias-pool tests may read the host."""
+        cores = list(cores)
+        if not cores:
+            raise ValueError("Hash3DAnchored routed gather: no tables")
+        c0 = cores[0]
+        for c in cores[1:]:
+            if c.local_size_ != c0.local_size_ or c.n_volumes_ != c0.n_volumes_:
+                raise ValueError(f"Hash3DAnchored routed gather: tables of local_size / n_volumes {c.local_size_} / "
+                                 f"{c.n_volumes_} and {c0.local_size_} / {c0.n_volumes_}; all must agree")
+        rows = [[c.shadow(force=recast).data_ptr(), c.prim_pool_.data_ptr(), _lib.ptr(c._bias()) or 0] for c in cores]
+        # an ordinary host-to-device copy, ordered on the current stream
+        return torch.tensor(rows, dtype=torch.int64).to(device, non_blocking=True)
+
+    @staticmethod
+    def launch_forward_residual_routed(cores, points, anchors, base_f16, ray_id, ray_table, out_f16=None, d_n_ptr=None,
+                                       refs=None, recast=True):
+        """out_f16 = base_f16 + cores[ray_table[ray_id[i]]].encode(points[i]) per sample, bit for bit what
+        `launch_forward_residual` of that table computes; a table id outside [0, len(cores)) leaves the base row.
+        ray_id int32 [n], ray_table int32 [n_rays] (device).  refs: `table_refs(cores, ...)` made once by a caller that
+        launches many times (else built here, one host-to-device copy)."""
+        out_f16 = base_f16 if out_f16 is None else out_f16
+        assert ray_id.dtype == torch.int32 and ray_table.dtype == torch.int32
+        if refs is None:
+            refs = Hash3DAnchoredCore.table_refs(cores, points.device, recast=recast)
+        c0 = cores[0]
+        with torch.cuda.device(points.device):
+            _lib.check(_lib.lib().gf_hash_forward_residual_routed(
+                points.shape[0], _lib.ptr(d_n_ptr), c0.n_volumes_, c0.local_size_, len(cores), _lib.ptr(refs),
+                _lib.ptr(c0.level_scales_), _lib.ptr(points), _lib.ptr(anchors), int(anchors.dtype == torch.int64),
+                _lib.ptr(ray_id), _lib.ptr(ray_table), _lib.ptr(base_f16), _lib.ptr(out_f16), _lib.cur_stream()),
+                "gf_hash_forward_residual_routed")
+
     def launch_backward(self, points, anchors, grad_in, grad_is_scaled_f16, grad_table, d_n_ptr=None,
                         keep_x128=False, levels=(0, 16)):
         """keep_x128: leave grad_table at the reference's x128 gradient scale (Hash3DAnchored_cuda.cu:209) for a

@@ -42,7 +42,7 @@ def _aligned(t: torch.Tensor) -> torch.Tensor:
     return t if t.data_ptr() % 16 == 0 else t.clone()
 
 
-def evaluate_views(model, cameras, images, camera_indices: Optional[Sequence[int]] = None
+def evaluate_views(model, cameras, images, camera_indices: Optional[Sequence[int]] = None, route_blocks: bool = False
                    ) -> Tuple[Dict[str, float], List[Dict[str, float]]]:
     """The body of nerfstudio's `Pipeline.get_average_eval_image_metrics` (nerfstudio/pipelines/base_pipeline.py)
     without the datamanager.  `cameras`: a `Cameras` with `width` and `height` set; `images`: one ground truth per
@@ -51,7 +51,8 @@ def evaluate_views(model, cameras, images, camera_indices: Optional[Sequence[int
     `model.get_outputs_for_camera_ray_bundle` -> `model.get_image_metrics_and_images`, plus `num_rays_per_sec`
     = H * W / wall time and `fps` = 1 / wall time, host clock from the render to the metrics' `.item()`.  The bundle
     has no `rel_camera_indices`: the model picks the appearance embedding by its nearest-camera rule, as the
-    reference's evaluation does.  Returns (averages: the mean of every key plus `psnr_std` and `ssim_std`, the
+    reference's evaluation does.  route_blocks: passed to `get_outputs_for_camera_ray_bundle` (a focal-stage model
+    evaluated with every chunk's own block table).  Returns (averages: the mean of every key plus `psnr_std` and `ssim_std`, the
     unbiased std of torch.std_mean as nerfstudio reports it; per_image: one dict per view)."""
     from .rays import RayBundle
     idx = list(range(len(cameras))) if camera_indices is None else [int(i) for i in camera_indices]
@@ -70,7 +71,7 @@ def evaluate_views(model, cameras, images, camera_indices: Optional[Sequence[int
                            metadata=rays.metadata)
         torch.cuda.synchronize(rays.origins.device)
         t0 = time.perf_counter()
-        outputs = model.get_outputs_for_camera_ray_bundle(bundle)
+        outputs = model.get_outputs_for_camera_ray_bundle(bundle, route_blocks=route_blocks)
         metrics, _ = model.get_image_metrics_and_images(outputs, {"image": gt})
         dt = time.perf_counter() - t0
         metrics["num_rays_per_sec"] = H * W / dt

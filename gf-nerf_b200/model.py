@@ -4,6 +4,7 @@ field -> get_weights_f2nerf -> RGB / depth / accumulation renderers -> octree fe
 `engine.GFNeRFEngine` is the same computation fused end to end on the compact layout (what bench.py times).
 `get_outputs_for_camera_ray_bundle` renders whole views of the modules' parameters through that fused path.
 """
+import os
 from typing import Dict, Tuple
 
 import torch
@@ -12,6 +13,7 @@ from torch import nn
 from . import _lib
 from .engine import FusedRenderer
 from .field import FieldHeadNames, GFNeRFField
+from .hash_3d_anchored import Hash3DAnchoredCore
 from .metrics import image_metrics
 from .perssampler import PersSampler
 from .rays import RayBundle
@@ -58,7 +60,8 @@ class GFNeRFModel(nn.Module):
     EVAL_NUM_RAYS_PER_CHUNK = 2048
 
     @torch.no_grad()
-    def get_outputs_for_camera_ray_bundle(self, camera_ray_bundle: RayBundle, chunk: int = 32768) -> Dict[str, torch.Tensor]:
+    def get_outputs_for_camera_ray_bundle(self, camera_ray_bundle: RayBundle, chunk: int = 32768,
+                                          route_blocks: bool = False) -> Dict[str, torch.Tensor]:
         """nerfstudio's `Model.get_outputs_for_camera_ray_bundle` (nerfstudio/models/base_model.py:166-190) on the fused
         kernels: `get_outputs` in eval mode over a whole view, `chunk` rays per fused render with no host sync in
         between.  origins / directions are [H, W, 3] (any leading shape works); returns {"rgb": [H,W,3],
@@ -70,8 +73,19 @@ class GFNeRFModel(nn.Module):
         optimizer state is made.  Rays take the embedding row of `rel_camera_indices` if the bundle has them, else
         the one of the training camera nearest to the first origin of their 2048-ray chunk, as the reference's
         `PersSampler.generate_ray_samples` chooses it for each `get_outputs` call of its evaluation loop.  The octree
-        is not updated and `self.training` is left as it is; the march noise follows the sampler's mode."""
+        is not updated and `self.training` is left as it is; the march noise follows the sampler's mode.
+
+        route_blocks (block stage only): every 2048-ray chunk adds the residual table of ITS block instead of the one
+        of `active_block_idxs_test` -- the block of the training camera nearest to the chunk's first origin, as the
+        reference's `generate_ray_samples` / `update_active_blocks(cur_split_dataset_idx)` choose it: the camera's
+        `cameras_labels` entry, else its index bucket.  The block follows the origins even when the bundle has
+        `rel_camera_indices`.  A block table that is not resident is loaded from `base_dir` (`load_table`) and stays
+        resident; one that is neither resident nor saved raises FileNotFoundError before anything is rendered.  The
+        fused chunks keep their size whatever the routes: the table is chosen per ray on the device."""
         f, rb = self.field, camera_ray_bundle
+        if route_blocks and f.cur_stage != "block_stage":
+            raise ValueError("get_outputs_for_camera_ray_bundle: route_blocks needs the block stage "
+                             f"(the field is in {f.cur_stage})")
         shape = tuple(rb.origins.shape[:-1])
         _lib.require_cuda(rb.origins, rb.directions)
         o = rb.origins.reshape(-1, 3).contiguous().float()
@@ -80,16 +94,22 @@ class GFNeRFModel(nn.Module):
         r = self._fused
         if r is None or r.sampler is not self.persampler.sampler or r.hidden != f.hidden_dim:
             r = self._fused = FusedRenderer(self.persampler.sampler, f.hidden_dim)
-        r.enc, r.res = f.base_encoding_init.hash_3d, None
-        if f.cur_stage == "block_stage":
+        r.enc, r.res, r.res_tables = f.base_encoding_init.hash_3d, None, None
+        ray_table, tables = None, []
+        if route_blocks:
+            ray_table, blocks = self._route_blocks(o)
+            tables = [getattr(f, f"base_encoding_{b}").hash_3d for b in blocks]
+        elif f.cur_stage == "block_stage":
             if len(f.active_block_idxs_test) != 1:
                 raise RuntimeError(f"get_outputs_for_camera_ray_bundle: the block stage renders one block table, "
                                    f"active_block_idxs_test is {f.active_block_idxs_test}")
             r.res = getattr(f, f"base_encoding_{f.active_block_idxs_test[0]}").hash_3d
-        for enc in (r.enc, r.res):
+        for enc in [r.enc, r.res] + tables:
             if enc is not None:
                 enc.shadow(force=True)
                 enc._bias()          # the all-zero test of the bias pool (a host read) before the chunk loop
+        if tables:
+            r.res_tables = (tables, Hash3DAnchoredCore.table_refs(tables, r.device, recast=False))
         blob = torch.cat([f.base_network.flat_params(), f.mlp_head.flat_params()]).float()
         if r.mlp is None or r.mlp.numel() != blob.numel():
             # the MLP kernels load a 16-byte vector tail past the blob (as for GFNeRFEngine.mlp)
@@ -102,7 +122,7 @@ class GFNeRFModel(nn.Module):
                 cam = rb.rel_camera_indices.reshape(n, -1)[:, 0].to(device=r.device, dtype=torch.int64)
             else:
                 cam = self._nearest_cameras(o)
-        rgb, depth, acc, first = r.render_rays(o, d, cam, chunk=chunk, first_oct_dis=True)
+        rgb, depth, acc, first = r.render_rays(o, d, cam, chunk=chunk, first_oct_dis=True, ray_table=ray_table)
         return {"rgb": rgb.view(*shape, 3), "accumulation": acc.view(*shape, 1),
                 "depth": (depth / self.scale_factor).view(*shape, 1),
                 "oct_depth": (first / self.scale_factor).view(*shape, 1)}
@@ -110,12 +130,44 @@ class GFNeRFModel(nn.Module):
     def _nearest_cameras(self, origins: torch.Tensor) -> torch.Tensor:
         """int64 [N]: per ray, the training camera nearest to the first origin of its EVAL_NUM_RAYS_PER_CHUNK-ray chunk,
         with the distance and argmin of `PersSampler.get_nearest_split_dataset*`; on the device, no host read."""
-        k = self.EVAL_NUM_RAYS_PER_CHUNK
+        return self._per_ray(self._chunk_nearest(origins), origins.shape[0]).to(origins.device)
+
+    def _chunk_nearest(self, origins: torch.Tensor) -> torch.Tensor:
+        """int64 [chunks]: the training camera nearest to the first origin of each EVAL_NUM_RAYS_PER_CHUNK-ray chunk"""
         c2w = self.persampler.c2w
-        firsts = origins[::k].to(c2w.device)                                        # [chunks, 3]
+        firsts = origins[::self.EVAL_NUM_RAYS_PER_CHUNK].to(c2w.device)                # [chunks, 3]
         dists = torch.linalg.norm(c2w[None, :, 0:3, -1] - firsts[:, None, :], dim=2)   # [chunks, cameras]
-        nearest = torch.argmin(dists, dim=1)
-        return nearest.view(-1, 1).expand(-1, k).reshape(-1)[:origins.shape[0]].to(origins.device)
+        return torch.argmin(dists, dim=1)
+
+    def _per_ray(self, per_chunk: torch.Tensor, n: int) -> torch.Tensor:
+        k = self.EVAL_NUM_RAYS_PER_CHUNK
+        return per_chunk.view(-1, 1).expand(-1, k).reshape(-1)[:n]
+
+    def _route_blocks(self, origins: torch.Tensor):
+        """(ray_table int32 [N], blocks): every ray's entry in `blocks`, the sorted block indices the view needs.  The
+        block of a chunk is `get_nearest_split_dataset*`'s: cameras_labels[nearest], or without labels
+        min(nearest // max(n_cams // n_split_dataset, 1), n_split_dataset - 1).  One host read (the block set); every
+        block's table is made resident here, or FileNotFoundError is raised before anything is launched."""
+        ps, f = self.persampler, self.field
+        nearest = self._chunk_nearest(origins)
+        if ps.cameras_labels is not None:
+            block = ps.cameras_labels.reshape(-1).to(nearest.device)[nearest].to(torch.int64)
+        else:
+            per = max(ps.c2w.shape[0] // ps.n_split_dataset, 1)
+            block = torch.clamp(nearest // per, max=ps.n_split_dataset - 1)
+        uniq = torch.unique(block)                                     # sorted
+        blocks = [int(b) for b in uniq.tolist()]                       # the call's one host read of the routes
+        missing = [b for b in blocks if not hasattr(f, f"base_encoding_{b}")]
+        for b in missing:
+            path = str(f.encodings_ckpt_dir / f"base_encoding_{b}.ckpt")
+            if not os.path.exists(path):
+                raise FileNotFoundError(f"block {b} has neither a resident table nor a saved one: {path}")
+        for b in missing:             # swapped out: brought back like update_active_blocks' eval branch does
+            f.load_table(b, strict=True)
+            getattr(f, f"base_encoding_{b}").set_require_grad(False)
+        slot = torch.searchsorted(uniq, block).to(torch.int32)
+        ray_table = self._per_ray(slot, origins.shape[0]).to(origins.device).contiguous()
+        return ray_table, blocks
 
     def get_image_metrics_and_images(self, outputs: Dict[str, torch.Tensor],
                                      batch: Dict[str, torch.Tensor]) -> Tuple[Dict[str, float], Dict[str, torch.Tensor]]:

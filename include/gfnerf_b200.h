@@ -92,6 +92,25 @@ int gf_hash_forward_residual(int64_t n, const int32_t* d_n_ptr, int32_t n_volume
                              const float* level_scales, const float* pts, const void* anchors, int anchor_i64,
                              const void* base_f16, void* out_f16, void* stream);
 
+/* One residual table of gf_hash_forward_residual_routed: its fp16 shadow, prime pool and bias pool (NULL = zeros).
+ * Every Hash3DAnchored draws its own primes, so each table carries its own pools. */
+typedef struct {
+  const void* feat_f16;
+  const int32_t* prim_pool;
+  const float* bias_pool;
+} gf_hash_table_ref;
+
+/* gf_hash_forward_residual with one of n_tables residual tables per sample: sample i adds table
+ * t = ray_table[ray_id[i]] of d_tables (a DEVICE array of n_tables descriptors), bit for bit what
+ * gf_hash_forward_residual computes with that table.  A t outside [0, n_tables) leaves the sample's base_f16 row
+ * unchanged in out_f16.  All tables share local_size and n_volumes.  ray_id: int32 [n], ray_table: int32 [n_rays].
+ * The focal stage's evaluation: each chunk of a view takes the block of its nearest training camera, and the routes
+ * stay on the device, so a fused render chunk may span several blocks. */
+int gf_hash_forward_residual_routed(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes, int64_t local_size,
+                                    int32_t n_tables, const gf_hash_table_ref* d_tables, const float* level_scales,
+                                    const float* pts, const void* anchors, int anchor_i64, const int32_t* ray_id,
+                                    const int32_t* ray_table, const void* base_f16, void* out_f16, void* stream);
+
 /* grad_in: fp32 [n,32] dL/dout (unscaled; grad_in_is_scaled_f16=0) -- the kernel
  * applies the reference's x128 -> fp16 quantisation (:209) -- or __half [n,32]
  * already scaled by 128 (grad_in_is_scaled_f16=1, produced by gf_mlp_backward).
