@@ -12,7 +12,7 @@ from .metrics import evaluate_views, image_metrics  # noqa: F401
 from .mlp import MLPNetwork  # noqa: F401
 from .model import GFNeRFModel  # noqa: F401
 from .cameras import Cameras  # noqa: F401
-from .pixel_samplers import ErrorPixelSampler, update_error_map  # noqa: F401
+from .pixel_samplers import ErrorPixelSampler, FocalBatchSource, update_error_map  # noqa: F401
 from .rays import Frustums, RayBundle, RaySamples, WarpedSamples  # noqa: F401
 from .renderers import AccumulationRenderer, DepthRenderer, RGBRenderer  # noqa: F401
 

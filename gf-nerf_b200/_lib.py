@@ -74,8 +74,14 @@ _SIGS = {
     "gf_adam_step": [_i64, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _i64, _f32, _int, _vp],
     "gf_image_metrics": [_i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp],
     "gf_image_metrics_scratch_bytes": [_i64, _i64, _i64],
+    "gf_sumtree_nodes": [_i64],
+    "gf_sumtree_build": [_i64, _vp, _vp, _vp, _vp],
+    "gf_sumtree_refresh": [_i64, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp],
+    "gf_focal_draw": [_i64, _i64, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i32, _i64,
+                      _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
 }
-_RET_I64 = ("gf_mlp_param_count", "gf_octree_proc_device_scratch_bytes", "gf_image_metrics_scratch_bytes")
+_RET_I64 = ("gf_mlp_param_count", "gf_octree_proc_device_scratch_bytes", "gf_image_metrics_scratch_bytes",
+            "gf_sumtree_nodes")
 
 EXPORTS = ["gf_last_error", "gf_version", "gf_launch_count", "gf_mlp_param_count", "gf_mlp_mask_words",
            "gf_octree_proc_device_scratch_bytes"] + sorted(_SIGS)

@@ -498,6 +498,35 @@ int gf_error_map_update(int64_t n_rays, const int64_t* indices, const float* pre
                         int64_t n_images, int64_t height, int64_t width, float* error_map, float* error_out,
                         int32_t* bad_index_flag, void* stream);
 
+/* ---- focal-stage batch source (csrc/focal_batch.cu) -----------------------
+ * Sum tree over a flat f32 error map of n pixels: fp64 sums and int32 counts of pixels > 0, gf_sumtree_nodes(n)
+ * entries each.  Level 0 = tiles of 1024 pixels, levels 1 and 2 = 32 children, level 3 = 16 children: one node per
+ * 2^24-pixel chunk.  Every node is a warp scan of its children in a fixed order, so a rebuild gives the same bits.
+ * gf_sumtree_refresh recomputes, from the map, the nodes above the pixels of n_rows (image, y, x) rows (i64 [n,3]);
+ * out-of-range rows are skipped.  The map must be 16-byte aligned. */
+int64_t gf_sumtree_nodes(int64_t n_pixels);
+int gf_sumtree_build(int64_t n_pixels, const float* error_map, double* sums, int32_t* counts, void* stream);
+int gf_sumtree_refresh(int64_t n_rows, const int64_t* indices, int64_t n_images, int64_t height, int64_t width,
+                       const float* error_map, double* sums, int32_t* counts, void* stream);
+
+/* One batch of ErrorPixelSampler.sample_method's distribution, drawn on the device without a host read.
+ * jobs: i64 [n_jobs, 10] = (lo, hi, count, weighted, chunk, cand_off, cand_cap, out_off, tab_off, tab_cap): `count`
+ * distinct pixels of [lo, hi) in successive-sampling order -- in proportion to the map over tree chunk `chunk` if
+ * weighted, else uniformly -- written to sel[out_off ...].  slot_job: i32 [total_cap], the job of each candidate slot;
+ * cand: i64 [total_cap]; tab_keys / tab_pos: the jobs' hash tables (tab_cap a power of two >= 2 (count + cand_cap));
+ * work: i32 [n_jobs + 1]; rng: i64 [2] = (Philox seed, counter), the counter advances by `rounds` on the device.
+ * Each of the `rounds` rounds draws with replacement and keeps first occurrences; finished jobs end the rounds early.
+ * Then the n_rows rows of sel become slot_out / idx_out (i64 [n,3], slot resp. image_idx[slot] in column 0),
+ * rel_out = rel_idx[slot], cam_out = image_idx[slot], rgb_out = images[slot, y, x], coords_out = (y + .5, x + .5).
+ * err (i32, caller zeroes) gets bit 1 for a chunk with fewer pixels > 0 than its count, bit 2 for a non-finite chunk
+ * sum, bit 4 for a job unfinished after `rounds`; the affected rows then hold in-range pixels of no meaning. */
+int gf_focal_draw(int64_t n_images, int64_t height, int64_t width, const float* error_map, const double* sums,
+                  const int32_t* counts, int64_t n_jobs, const int64_t* jobs, const int32_t* slot_job,
+                  int64_t total_cap, int64_t* cand, uint64_t* tab_keys, int32_t* tab_pos, int32_t* work,
+                  int64_t* rng, int32_t rounds, int64_t n_rows, int64_t* sel, const float* images,
+                  const int64_t* image_idx, const int64_t* rel_idx, int64_t* slot_out, int64_t* idx_out,
+                  int64_t* rel_out, float* rgb_out, float* coords_out, int64_t* cam_out, int32_t* err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
