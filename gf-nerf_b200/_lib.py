@@ -31,6 +31,7 @@ _SIGS = {
                                         _vp],
     "gf_hash_backward": [_i64, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _int, _vp, _vp],
     "gf_hash_backward_levels": [_i64, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _int, _vp, _int, _int, _vp],
+    "gf_hash_backward_routed": [_i64, _vp, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp, _int, _vp],
     "gf_hash_corner_rows": [_i64, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _int, _vp, _vp],
     "gf_sampler_get_samples": [_i64, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _f32, _f32, _int, _i64,
                                C.POINTER(SamplerOut), _vp],

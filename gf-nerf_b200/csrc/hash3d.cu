@@ -210,13 +210,50 @@ hash_fwd_routed_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n
                                                       anchors, out16, nullptr, base16);
 }
 
-template <bool POW2, typename AnchorT, bool GRAD_F16, bool HAS_BIAS, bool UNSCALE>
-__global__ void __launch_bounds__(kHashBlock, 4)   // 64 registers: four CTAs per SM (three at 72 cost 4 %, r02z)
-hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes, uint32_t local_size,
-                const int32_t* __restrict__ prim_pool, const float* __restrict__ bias_pool,
-                const float* __restrict__ scales, const float* __restrict__ pts,
-                const AnchorT* __restrict__ anchors, const void* __restrict__ grad_in_v,
-                float* __restrict__ grad_table, int level_begin, int level_end) {
+// The table a sample's gradient goes to.  `OneGradTable`: every sample the same (hash_bwd_kernel).  `RoutedGradTables`:
+// sample i takes table ray_table[ray_id[i]] of a device descriptor array (hash_bwd_routed_kernel); an id outside
+// [0, n_tables) contributes nothing (the lane is treated like one past the end, with table 0's pools for its
+// unused cell, and a run key of its own).  `key` is the table id that, with the volume, starts a new run.
+struct OneGradTable {
+  static constexpr bool kRouted = false;
+  const int32_t* __restrict__ prim_pool;
+  const float* __restrict__ bias_pool;
+  float* __restrict__ grad_table;
+  __device__ __forceinline__ bool operator()(int64_t, bool, const int32_t*& p, const float*& b, float*& g,
+                                             int32_t&) const {
+    p = prim_pool;
+    b = bias_pool;
+    g = grad_table;
+    return true;
+  }
+};
+
+struct RoutedGradTables {
+  static constexpr bool kRouted = true;
+  const gf_hash_grad_ref* __restrict__ tables;
+  int32_t n_tables;
+  const int32_t* __restrict__ ray_id;
+  const int32_t* __restrict__ ray_table;
+  __device__ __forceinline__ bool operator()(int64_t i, bool valid, const int32_t*& p, const float*& b, float*& g,
+                                             int32_t& key) const {
+    const int32_t t = valid ? __ldg(ray_table + __ldg(ray_id + i)) : -1;
+    const bool ok = (uint32_t)t < (uint32_t)n_tables;
+    key = ok ? t : -1;
+    const gf_hash_grad_ref* r = tables + (ok ? t : 0);
+    p = reinterpret_cast<const int32_t*>(__ldg(reinterpret_cast<const unsigned long long*>(&r->prim_pool)));
+    b = reinterpret_cast<const float*>(__ldg(reinterpret_cast<const unsigned long long*>(&r->bias_pool)));
+    g = reinterpret_cast<float*>(__ldg(reinterpret_cast<const unsigned long long*>(&r->grad_table)));
+    return ok;
+  }
+};
+
+// The backward scatter of hash_bwd_kernel and hash_bwd_routed_kernel: a warp per 32 consecutive samples, all levels.
+template <bool POW2, typename AnchorT, bool GRAD_F16, bool HAS_BIAS, bool UNSCALE, typename Tables>
+__device__ __forceinline__ void hash_bwd_body(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes,
+                                              uint32_t local_size, const Tables& tables,
+                                              const float* __restrict__ scales, const float* __restrict__ pts,
+                                              const AnchorT* __restrict__ anchors, const void* __restrict__ grad_in_v,
+                                              int level_begin, int level_end) {
   if (d_n_ptr) {
     int64_t dn = *d_n_ptr;
     n = dn < n ? dn : n;
@@ -232,12 +269,17 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
   if (threadIdx.x < GF_N_LEVELS) s_scale[threadIdx.x] = __ldg(scales + threadIdx.x);
   __syncthreads();
   const int lane = lane_id();
-  uint32_t* sg = s_grad + (GRAD_F16 ? (threadIdx.x >> 5) * 32 * kGradRowWords : 0);
+  // (the mask restates the kernels' launch bounds, which the compiler no longer applies here after inlining)
+  uint32_t* sg = s_grad + (GRAD_F16 ? ((threadIdx.x & (kHashBlock - 1)) >> 5) * 32 * kGradRowWords : 0);
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   // warp-uniform trip count: every lane of a warp runs the same iterations
   for (int64_t base = (int64_t)blockIdx.x * blockDim.x + threadIdx.x - lane; base < n; base += stride) {
     const int64_t i = base + lane;
-    const bool valid = i < n;
+    const int32_t* prim_pool;
+    const float* bias_pool;
+    float* grad_table;
+    int32_t key = 0;
+    const bool valid = tables(i, i < n, prim_pool, bias_pool, grad_table, key) && i < n;
     float x = 0.f, y = 0.f, z = 0.f;
     int vol = 0;
     if (valid) {
@@ -247,7 +289,11 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
       vol = (int)anchors[i];
     }
     const int pvol = __shfl_up_sync(0xffffffffu, vol, 1);  // by all 32 lanes: not inside the || below
-    const bool vol_head = lane == 0 || pvol != vol;
+    bool vol_head = lane == 0 || pvol != vol;
+    if (Tables::kRouted) {  // a run also ends where the table changes
+      const int32_t pkey = __shfl_up_sync(0xffffffffu, key, 1);   // by all 32 lanes, like pvol
+      vol_head = vol_head || pkey != key;
+    }
     if (GRAD_F16) {
       __syncwarp();  // the previous batch's readers are done with sg
       const uint4* src = reinterpret_cast<const uint4*>(grad_in_v) + base * (GF_N_LEVELS / 4);
@@ -269,17 +315,48 @@ hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volume
       __half2 gh = __float2half2_rn(0.f);
       if (GRAD_F16) {
         gh = *reinterpret_cast<const __half2*>(sg + lane * kGradRowWords + l);   // (rows past the end were zero-filled)
+        if (Tables::kRouted && !valid) gh = __float2half2_rn(0.f);            // (a sample routed to no table)
       } else if (valid) {
         {
           const float2 v = __ldg(reinterpret_cast<const float2*>(grad_in_v) + i * GF_N_LEVELS + l);
           gh = __floats2half2_rn(__fmul_rn(v.x, GF_GRAD_SCALE), __fmul_rn(v.y, GF_GRAD_SCALE));
         }
       }
-      hash_scatter_level<POW2, HAS_BIAS, UNSCALE>(l, x, y, z, vol, vol_head, gh, lane, n_volumes, local_size, prim_pool,
-                                                  bias_pool, s_scale[l], grad_table,
-                                                  s_stage + (threadIdx.x >> 5) * kScatterWarpWords);
+      hash_scatter_level<POW2, HAS_BIAS, UNSCALE, Tables::kRouted>(
+          l, x, y, z, vol, vol_head, gh, lane, n_volumes, local_size, prim_pool, bias_pool, s_scale[l], grad_table,
+          s_stage + (threadIdx.x >> 5) * kScatterWarpWords);
     }
   }
+}
+
+template <bool POW2, typename AnchorT, bool GRAD_F16, bool HAS_BIAS, bool UNSCALE>
+__global__ void __launch_bounds__(kHashBlock, 4)   // 64 registers: four CTAs per SM (three at 72 cost 4 %, r02z)
+hash_bwd_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes, uint32_t local_size,
+                const int32_t* __restrict__ prim_pool, const float* __restrict__ bias_pool,
+                const float* __restrict__ scales, const float* __restrict__ pts,
+                const AnchorT* __restrict__ anchors, const void* __restrict__ grad_in_v,
+                float* __restrict__ grad_table, int level_begin, int level_end) {
+  hash_bwd_body<POW2, AnchorT, GRAD_F16, HAS_BIAS, UNSCALE>(n, d_n_ptr, n_volumes, local_size,
+                                                            OneGradTable{prim_pool, bias_pool, grad_table}, scales,
+                                                            pts, anchors, grad_in_v, level_begin, level_end);
+}
+
+// Scatter with a gradient table per sample (gf_hash_backward_routed), all 16 levels.  A table's bias pool is read
+// when its descriptor has one (a per-lane test instead of the HAS_BIAS instantiation).
+// Registers: the three per-lane table pointers fit the 64 of four CTAs per SM when the table stays at the x128 scale
+// Registers: with the three per-lane table pointers, the variant that leaves the table at the x128 scale (the engine's
+// call) spills at the 64 registers of four CTAs per SM (ptxas keeps the unscaled variant's multiplier in a register
+// and schedules differently), so it runs three at up to 80; the unscaled variant fits 64 and keeps four.
+template <bool POW2, typename AnchorT, bool GRAD_F16, bool UNSCALE>
+__global__ void __launch_bounds__(kHashBlock, UNSCALE ? 4 : 3)
+hash_bwd_routed_kernel(int64_t n, const int32_t* __restrict__ d_n_ptr, int32_t n_volumes, uint32_t local_size,
+                       int32_t n_tables, const gf_hash_grad_ref* __restrict__ tables,
+                       const float* __restrict__ scales, const float* __restrict__ pts,
+                       const AnchorT* __restrict__ anchors, const int32_t* __restrict__ ray_id,
+                       const int32_t* __restrict__ ray_table, const void* __restrict__ grad_in_v) {
+  hash_bwd_body<POW2, AnchorT, GRAD_F16, false, UNSCALE>(n, d_n_ptr, n_volumes, local_size,
+                                                         RoutedGradTables{tables, n_tables, ray_id, ray_table}, scales,
+                                                         pts, anchors, grad_in_v, 0, GF_N_LEVELS);
 }
 
 // table row of every corner, int32 [n,16,8] -- the parity probe for "bit-exact hash indices"
@@ -492,6 +569,48 @@ int gf_hash_backward_levels(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes
 #undef GF_BWD_U
 #undef GF_BWD
   return check_launch("hash_bwd_kernel");
+}
+
+int gf_hash_backward_routed(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes, int64_t local_size,
+                            int32_t n_tables, const gf_hash_grad_ref* d_tables, const float* level_scales,
+                            const float* pts, const void* anchors, int anchor_i64, const int32_t* ray_id,
+                            const int32_t* ray_table, const void* grad_in, int grad_in_is_scaled_f16, void* stream) {
+  GF_REQUIRE(n >= 0 && n_volumes > 0 && local_size > 0 && local_size <= 0x7fffffffLL && local_size % 2 == 0,
+             "gf_hash_backward_routed: bad sizes n=%lld n_volumes=%d local_size=%lld (must be even)", (long long)n,
+             n_volumes, (long long)local_size);
+  GF_REQUIRE(n_tables > 0, "gf_hash_backward_routed: n_tables = %d (must be > 0)", n_tables);
+  GF_REQUIRE(d_tables && ray_id && ray_table, "gf_hash_backward_routed: null table descriptors / ray_id / ray_table");
+  if (n == 0) return GF_OK;
+  GF_REQUIRE(level_scales && pts && anchors && grad_in, "gf_hash_backward_routed: null pointer");
+  GF_REQUIRE((reinterpret_cast<uintptr_t>(grad_in) & 15) == 0,
+             "gf_hash_backward_routed: grad_in must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int grid = stride_grid(n, kHashBlock, 4, 4);
+  const bool p2 = is_pow2(local_size);
+  const bool g16 = (grad_in_is_scaled_f16 & 1) != 0, unscale = (grad_in_is_scaled_f16 & 2) == 0;
+#define GF_BWD_R(P2, AT, G16, US)                                                                               \
+  hash_bwd_routed_kernel<P2, AT, G16, US><<<grid, kHashBlock, 0, st>>>(                                         \
+      n, d_n_ptr, n_volumes, (uint32_t)local_size, n_tables, d_tables, level_scales, pts, (const AT*)anchors,   \
+      ray_id, ray_table, grad_in)
+#define GF_BWD_RU(P2, AT, G16)                      \
+  do {                                              \
+    if (unscale) GF_BWD_R(P2, AT, G16, true);       \
+    else GF_BWD_R(P2, AT, G16, false);              \
+  } while (0)
+#define GF_BWD_RG(P2, AT)                           \
+  do {                                              \
+    if (g16) GF_BWD_RU(P2, AT, true);               \
+    else GF_BWD_RU(P2, AT, false);                  \
+  } while (0)
+  if (p2) {
+    if (anchor_i64) GF_BWD_RG(true, int64_t); else GF_BWD_RG(true, int32_t);
+  } else {
+    if (anchor_i64) GF_BWD_RG(false, int64_t); else GF_BWD_RG(false, int32_t);
+  }
+#undef GF_BWD_RG
+#undef GF_BWD_RU
+#undef GF_BWD_R
+  return check_launch("hash_bwd_routed_kernel");
 }
 
 int gf_hash_corner_rows(int64_t n, int32_t n_volumes, int64_t local_size, const int32_t* prim_pool,

@@ -119,7 +119,11 @@ __device__ __forceinline__ void red_add_f32x2(float2* tab, uint32_t row, float s
 // in another volume (the same at every level, so the caller shuffles it once).  Must be called by all 32 lanes.
 // UNSCALE: the sums are divided by GF_GRAD_SCALE (:238); false leaves the table at the x128 scale for a caller that
 // folds the division into its optimizer step (exact either way: a power of two).
-template <bool POW2, bool HAS_BIAS, bool UNSCALE>
+// ROUTED: prim_pool, bias_pool (NULL = zeros, HAS_BIAS ignored) and grad_table are this lane's table's, which may differ
+// between lanes; the caller's vol_head then also starts a run where the table changes.  The shared-memory walker keeps
+// each lane's level base pointer in the two spare words of its staging row and flushes a run through the pointer of
+// the lane that closes it; the shuffle paths flush from the run's first lane with its own pointer.
+template <bool POW2, bool HAS_BIAS, bool UNSCALE, bool ROUTED = false>
 __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, float z, int vol, bool vol_head, __half2 gh,
                                                    int lane, int32_t n_volumes, uint32_t local_size,
                                                    const int32_t* __restrict__ prim_pool,
@@ -128,7 +132,8 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
   // every product of a zero gradient is zero and no reduction of this level would be issued
   if (!__any_sync(0xffffffffu, *reinterpret_cast<const uint32_t*>(&gh) & 0x7fff7fffu)) return;
   const int tr = (l * n_volumes + vol) * 3;
-  const Cell c = cell_of(x, y, z, scale, HAS_BIAS ? bias_pool + tr : nullptr);
+  const Cell c = cell_of(x, y, z, scale,
+                         ROUTED ? (bias_pool ? bias_pool + tr : nullptr) : HAS_BIAS ? bias_pool + tr : nullptr);
   const uint32_t pa = (uint32_t)__ldg(prim_pool + tr), pb = (uint32_t)__ldg(prim_pool + tr + 1),
                  pc = (uint32_t)__ldg(prim_pool + tr + 2);
   uint32_t pos[8];
@@ -158,6 +163,7 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
     uint2* row = reinterpret_cast<uint2*>(s_warp + lane * kScatterRowWords);
 #pragma unroll
     for (int d = 0; d < 8; d++) row[d] = make_uint2(cq[d], pos[d]);
+    if (ROUTED) *reinterpret_cast<float2**>(row + 8) = tab;   // words 16-17: 8-byte aligned (72-byte rows)
     __syncwarp();
     const int d = lane & 7, j0 = lane & 24;
     // bit k: lane j0 + k is the last of its run or of its quarter
@@ -170,7 +176,9 @@ __device__ __forceinline__ void hash_scatter_level(int l, float x, float y, floa
       a0 = k == 0 ? v.x : a0 + v.x;  // (not 0 + v: a -0 differs only in a zero sum, which is never written)
       a1 = k == 0 ? v.y : a1 + v.y;
       const bool stop = (stops >> k) & 1u;
-      red_add_f32x2<UNSCALE>(tab, e.y, a0, a1, stop ? kScatterKeep : 0u);
+      float2* const t =
+          ROUTED ? *reinterpret_cast<float2* const*>(s_warp + (j0 + k) * kScatterRowWords + 16) : tab;
+      red_add_f32x2<UNSCALE>(t, e.y, a0, a1, stop ? kScatterKeep : 0u);
       a0 = stop ? 0.f : a0;
       a1 = stop ? 0.f : a1;
     }

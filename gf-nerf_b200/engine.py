@@ -94,6 +94,7 @@ class StepOutputs:
     accumulation: torch.Tensor   # [R]
     loss: Optional[torch.Tensor]  # [1] or None
     n_samples: torch.Tensor      # int32 [1] (device)
+    block_losses: Optional[torch.Tensor] = None   # [K]: each block's loss (several focal blocks); loss is their sum
 
 
 class FusedRenderer:
@@ -361,26 +362,70 @@ class GFNeRFEngine(FusedRenderer):
         self._deferred = None   # lr_scale of an optimizer step whose gradient reduce is still in flight
         self.stage = "init_stage"
         self.opt_res = None     # focal stage: Adam of this GPU's residual sub-encoder `res`
+        # focal stage with several blocks (start_block_stage(blocks=...)): their ids, residual cores and Adams
+        self.blocks = self.res_blocks = self.opt_res_blocks = None
 
     # ---- focal (block) stage: reference gfnerf/nerfacto_field.py:458-489, gfnerf/nerfacto.py:432-488 ------------
-    def start_block_stage(self, log2_table_size: int = None, lr: float = 5e-3, seed: int = 1):
+    def start_block_stage(self, log2_table_size: int = None, lr: float = 5e-3, seed: int = 1, blocks=None):
         """Freezes the global table, both MLPs and the appearance embedding and adds a zero-initialised residual
-        sub-encoder whose features are summed with the global encoder's before the (frozen) MLP.  One block per GPU:
-        the residual table is private to this rank, so the focal stage has NO gradient exchange at all."""
+        sub-encoder whose features are summed with the global encoder's before the (frozen) MLP.  The residual tables
+        are private to this rank, so the focal stage has NO gradient exchange at all.
+
+        blocks = [b0, ..., bK-1]: this rank trains K blocks at once, table k seeded `seed + k` (the table a single-block
+        engine started with `seed + k` has).  A training batch is then K equal contiguous segments of rays, segment k
+        belonging to blocks[k]; each block's step is what a single-block engine computes on its segment.  Renders
+        take a per-ray `ray_table` (index into `blocks`).  Without `blocks`: one residual table `res`."""
+        if blocks is not None:
+            blocks = [int(b) for b in blocks]
+            if not blocks or len(set(blocks)) != len(blocks) or min(blocks) < 0:
+                raise ValueError(f"gfnerf_b200: block ids must be distinct and >= 0, got {blocks}")
         self.flush()
         log2_table_size = int(np.log2(self.enc.local_size_)) if log2_table_size is None else int(log2_table_size)
-        gen = torch.Generator().manual_seed(seed)
-        self.res = Hash3DAnchoredCore(log2_table_size, self.n_volumes, device=self.device, generator=gen)
-        self.res.feat_pool_.requires_grad_(False)
-        self.res.Zero()
-        self.res.shadow(force=True)
-        self.opt_res = _Adam(self.res.feat_pool_.detach().view(-1), lr, grad_scale=GRAD_SCALE,   # sub-encoder lr, gfnerf/nerfacto.py:483
-                             n_active=self.res.used_rows_ * 2)
+
+        def block_table(seed_):
+            res = Hash3DAnchoredCore(log2_table_size, self.n_volumes, device=self.device,
+                                     generator=torch.Generator().manual_seed(seed_))
+            res.feat_pool_.requires_grad_(False)
+            res.Zero()
+            res.shadow(force=True)
+            opt = _Adam(res.feat_pool_.detach().view(-1), lr, grad_scale=GRAD_SCALE,   # sub-encoder lr, gfnerf/nerfacto.py:483
+                        n_active=res.used_rows_ * 2)
+            return res, opt
+
+        self.res = self.opt_res = self.res_tables = None
+        self.blocks = self.res_blocks = self.opt_res_blocks = None
+        if blocks is None:
+            self.res, self.opt_res = block_table(seed)
+        else:
+            made = [block_table(seed + k) for k in range(len(blocks))]
+            self.blocks = blocks
+            self.res_blocks = [m[0] for m in made]
+            self.opt_res_blocks = [m[1] for m in made]
+            self._block_refs()
         self.stage = "block_stage"
         self.sampler.UpdateMode(1)                                        # nerfacto.py:614-616
 
+    def _block_refs(self):
+        """Descriptor arrays of the block tables for the routed gather and scatter (again after a pool was replaced)"""
+        self.res_tables = (self.res_blocks, Hash3DAnchoredCore.table_refs(self.res_blocks, self.device, recast=False))
+        self._grad_refs = Hash3DAnchoredCore.grad_refs(self.res_blocks, [o.grad for o in self.opt_res_blocks],
+                                                       self.device)
+        self._block_ray_tables = {}
+
+    def block_ray_table(self, n_rays: int) -> torch.Tensor:
+        """int32 [n_rays]: the training batch's route, K contiguous segments of n_rays / K rays, segment k to table k"""
+        K = len(self.blocks)
+        if n_rays % K:
+            raise ValueError(f"gfnerf_b200: a batch of {n_rays} rays does not split into {K} equal block segments")
+        rt = self._block_ray_tables.get(n_rays)
+        if rt is None:
+            rt = torch.arange(K, dtype=torch.int32, device=self.device).repeat_interleave(n_rays // K)
+            self._block_ray_tables[n_rays] = rt
+        return rt
+
     def end_block_stage(self):
-        self.res = self.opt_res = None
+        self.res = self.opt_res = self.res_tables = None
+        self.blocks = self.res_blocks = self.opt_res_blocks = None
         self.stage = "init_stage"
         self.sampler.UpdateMode(0)
 
@@ -431,18 +476,26 @@ class GFNeRFEngine(FusedRenderer):
     def store_model(self, model, block: Optional[int] = None):
         """The inverse of `load_model`: the engine's current parameters into the field's modules (whose `state_dict()`
         is the reference's checkpoint layout).  block = b (block stage only): the residual table `res` also goes into
-        the field's `base_encoding_{b}`, which is created if the field has none -- how the blocks of a focal run,
-        one per rank, are gathered into one model (each rank stores its block, then `field.save_table(b)`)."""
+        the field's `base_encoding_{b}`, which is created if the field has none -- how the blocks of a focal run
+        are gathered into one model (each rank stores its blocks, then `field.save_table(b)`).  With several blocks
+        (start_block_stage(blocks=...)) b must be one of them, and its table is the one stored."""
         f = getattr(model, "field", model)
         if int(f.hidden_dim) != self.hidden:
             raise ValueError(f"gfnerf_b200: the field is {f.hidden_dim} wide, the engine {self.hidden}")
+        res = None
         if block is not None:
-            if self.stage != "block_stage" or self.res is None:
+            if self.stage != "block_stage" or (self.res is None and self.blocks is None):
                 raise ValueError(f"gfnerf_b200: store_model(block={block}) needs the block stage; the engine is in "
                                  f"{self.stage}")
-            if int(f.log2_table_size) != int(np.log2(self.res.local_size_)):
+            if self.blocks is not None:
+                if int(block) not in self.blocks:
+                    raise ValueError(f"gfnerf_b200: block {block} is not one of this engine's blocks {self.blocks}")
+                res = self.res_blocks[self.blocks.index(int(block))]
+            else:
+                res = self.res
+            if int(f.log2_table_size) != int(np.log2(res.local_size_)):
                 raise ValueError(f"gfnerf_b200: the field's block tables are 2^{f.log2_table_size} rows per level, "
-                                 f"the engine's residual table 2^{int(np.log2(self.res.local_size_))}")
+                                 f"the engine's residual table 2^{int(np.log2(res.local_size_))}")
         self.flush()
         self.sync_master_params()       # peer exchange: every rank only keeps ITS fp32 rows current
         f.base_encoding_init.load_states([t.detach() for t in self.enc.States()], 0)
@@ -459,7 +512,7 @@ class GFNeRFEngine(FusedRenderer):
             name = f"base_encoding_{int(block)}"
             if not hasattr(f, name):
                 f.add_table(int(block))
-            getattr(f, name).load_states([t.detach() for t in self.res.States()], 0)
+            getattr(f, name).load_states([t.detach() for t in res.States()], 0)
 
     # ---- resume ---------------------------------------------------------------------------------------------------------
     def checkpoint(self) -> dict:
@@ -489,6 +542,11 @@ class GFNeRFEngine(FusedRenderer):
             out["res_table"] = [cpu(t) for t in self.res.States()]
             out["adam"]["res"] = adam(self.opt_res)
             out["res_lr"] = self.opt_res.lr
+        if self.blocks is not None:
+            out["res_blocks"] = list(self.blocks)
+            out["res_block_tables"] = [[cpu(t) for t in c.States()] for c in self.res_blocks]
+            out["adam"]["res_blocks"] = [adam(o) for o in self.opt_res_blocks]
+            out["res_lr"] = self.opt_res_blocks[0].lr
         return out
 
     def restore(self, ckpt: dict) -> None:
@@ -529,7 +587,16 @@ class GFNeRFEngine(FusedRenderer):
         s.UpdateMode(int(ss["mode"]))
         s._octree_stale = True                 # the host mirror picks the statistics up when somebody asks for it
         self.step_count = int(ckpt["step_count"])
-        if ckpt["stage"] == "block_stage":
+        if ckpt["stage"] == "block_stage" and "res_blocks" in ckpt:
+            tables = ckpt["res_block_tables"]
+            self.start_block_stage(log2_table_size=int(np.log2(tables[0][0].shape[0] // 16)),
+                                   lr=float(ckpt["res_lr"]), blocks=ckpt["res_blocks"])
+            for c, o, t, st in zip(self.res_blocks, self.opt_res_blocks, tables, ckpt["adam"]["res_blocks"]):
+                c.LoadStates(t, 0)
+                c.shadow(force=True)
+                adam(o, st)
+            self._block_refs()                 # LoadStates replaced the prime pools
+        elif ckpt["stage"] == "block_stage":
             self.start_block_stage(log2_table_size=int(np.log2(ckpt["res_table"][0].shape[0] // 16)),
                                    lr=float(ckpt["res_lr"]))
             self.res.LoadStates(ckpt["res_table"], 0)
@@ -678,8 +745,16 @@ class GFNeRFEngine(FusedRenderer):
     def train_step(self, rays_o, rays_d, target_rgb, rel_camera_indices=None, noise=None, lr_scale: float = 1.0,
                    update_octree: bool = True, optimizer_step: bool = True, next_rays=None) -> StepOutputs:
         """next_rays = (rays_o, rays_d) of the batch the NEXT call will be given: their sampling is started as soon
-        as this step's octree vote has been issued and overlaps this step's backward pass (`_presample`)."""
+        as this step's octree vote has been issued and overlaps this step's backward pass (`_presample`).
+
+        Several focal blocks (start_block_stage(blocks=...)): the batch is K equal contiguous segments, segment k
+        belonging to blocks[k].  The loss terms are computed per segment (S3IM's permutations stay inside it) and
+        returned in `block_losses`; `loss` is their sum.  One routed scatter takes every sample to its block's
+        gradient table, and each block has its own NaN guard and Adam step."""
         L = _lib.lib()
+        multi = self.stage == "block_stage" and self.blocks is not None
+        K = len(self.blocks) if multi else 1
+        ray_table = self.block_ray_table(rays_o.shape[0]) if multi else None
         with torch.cuda.device(self.device):
             st = _lib.cur_stream()
             step = self.step_count
@@ -689,23 +764,28 @@ class GFNeRFEngine(FusedRenderer):
             self.flush()   # a deferred optimizer step of the previous iteration lands here
             cap, R = cs.pts01.shape[0], cs.n_rays
             ray_emb = self._ray_emb(rel_camera_indices)
-            feat, sigma, rgb, ray_bias = self._field_forward(cs, ray_emb, train=True)
+            feat, sigma, rgb, ray_bias = self._field_forward(cs, ray_emb, train=True, ray_table=ray_table)
             out_rgb, depth, acc, weights, alphas, trans = self._composite(cs, sigma, rgb, keep=True)
             # loss (CharbonnierLoss, nerfstudio/model_components/losses.py:73-84)
             g_rgb = self._buf("g_rgb", (R, 3), torch.float32)
-            loss = torch.zeros(1, dtype=torch.float32, device=self.device)
             target = target_rgb.contiguous().float()
+            Rb = R // K
+            losses = torch.zeros(K, dtype=torch.float32, device=self.device)   # K = 1: the step's loss
             with self._stage("loss"):
-                _lib.check(L.gf_charbonnier(R, _lib.ptr(out_rgb), _lib.ptr(target), 1e-6,
-                                            _lib.ptr(g_rgb), _lib.ptr(loss), st), "gf_charbonnier")
+                for k in range(K):
+                    _lib.check(L.gf_charbonnier(Rb, _lib.ptr(out_rgb[k * Rb:]), _lib.ptr(target[k * Rb:]), 1e-6,
+                                                _lib.ptr(g_rgb[k * Rb:]), _lib.ptr(losses[k:]), st), "gf_charbonnier")
             mult, ks, stride, repeat, patch_h = self.s3im
-            if mult > 0.0 and (R * repeat) % patch_h == 0:
+            if mult > 0.0 and (Rb * repeat) % patch_h == 0:
                 # S3IM.forward (losses.py:779-794): the batch once in order, then repeat-1 random permutations
-                perms = torch.rand((repeat - 1, R), device=self.device).argsort(dim=1)
-                index = torch.cat([torch.arange(R, device=self.device).view(1, R), perms]).reshape(-1).contiguous()
-                with self._stage("loss"):
-                    _lib.check(L.gf_s3im(R, index.numel(), _lib.ptr(index), _lib.ptr(out_rgb), _lib.ptr(target),
-                                         patch_h, ks, stride, mult, _lib.ptr(g_rgb), _lib.ptr(loss), st), "gf_s3im")
+                perms = torch.rand((K, repeat - 1, Rb), device=self.device).argsort(dim=2)
+                for k in range(K):
+                    index = torch.cat([torch.arange(Rb, device=self.device).view(1, Rb), perms[k]]).reshape(-1).contiguous()
+                    with self._stage("loss"):
+                        _lib.check(L.gf_s3im(Rb, index.numel(), _lib.ptr(index), _lib.ptr(out_rgb[k * Rb:]),
+                                             _lib.ptr(target[k * Rb:]), patch_h, ks, stride, mult,
+                                             _lib.ptr(g_rgb[k * Rb:]), _lib.ptr(losses[k:]), st), "gf_s3im")
+            loss = losses.sum().view(1) if multi else losses
             # training feedback (gfnerf/nerfacto.py:598-616).  It only needs the forward's weights, so it is issued
             # here: its (tiny) MAX all-reduce over ranks must not queue behind the gradient all-reduce below
             vote = None
@@ -728,7 +808,7 @@ class GFNeRFEngine(FusedRenderer):
                                                    _lib.ptr(rgb), _lib.ptr(trans), _lib.ptr(g_rgb), None, None,
                                                    _lib.ptr(d_sigma), _lib.ptr(d_rgb), st), "gf_composite_backward")
             d_feat = self._buf("d_feat", (cap, 32), torch.float16)
-            grad_scale = float(2 ** int(np.ceil(np.log2(max(R, 1)))))
+            grad_scale = float(2 ** int(np.ceil(np.log2(max(Rb, 1)))))   # (per block: the single-block d_feat bits)
             block = self.stage == "block_stage"
             d_ray_bias = None if block else self._buf("d_ray_bias", (R, self.hidden), torch.float32, zero=True)
             with self._stage("mlp_bwd"):   # block stage: frozen MLP, only d_feat
@@ -742,7 +822,19 @@ class GFNeRFEngine(FusedRenderer):
                 # issued behind the MLP backward: that kernel is resident first (2 CTAs / SM, tensor pipe + epilogue,
                 # ~25 % of the issue slots) and the sampler's CTAs fill the registers it leaves free
                 self._presample(next_rays[0], next_rays[1], vote, after=fwd_done)
-            if block:
+            if multi:
+                with self._stage("hash_bwd"):
+                    Hash3DAnchoredCore.launch_backward_routed(self.res_blocks, cs.pts01, cs.anchor, d_feat, True,
+                                                              cs.ray_id, ray_table, refs=self._grad_refs,
+                                                              d_n_ptr=cs.total, keep_x128=True)
+                if optimizer_step:
+                    with self._stage("adam_table"):
+                        flags = self._nan_flags([o.grad[:o.n_active] for o in self.opt_res_blocks])
+                        for k, (res, opt) in enumerate(zip(self.res_blocks, self.opt_res_blocks)):
+                            opt.step(shadow=res._shadow, lr=opt.lr * lr_scale,
+                                     skip_flag=None if flags is None else flags[k:k + 1])
+                            res.mark_shadow_fresh()
+            elif block:
                 with self._stage("hash_bwd"):
                     self.res.launch_backward(cs.pts01, cs.anchor, d_feat, True, self.opt_res.grad.view(-1, 2),
                                              d_n_ptr=cs.total, keep_x128=True)
@@ -787,7 +879,7 @@ class GFNeRFEngine(FusedRenderer):
                     if optimizer_step:
                         self._reduce_and_step(lr_scale)
             self.step_count += 1
-        return StepOutputs(out_rgb, depth, acc, loss, cs.total)
+        return StepOutputs(out_rgb, depth, acc, loss, cs.total, losses if multi else None)
 
     # ---- host-buffer entry point ------------------------------------------------------------------------------
     @torch.no_grad()
@@ -908,6 +1000,18 @@ class GFNeRFEngine(FusedRenderer):
             _lib.check(L.gf_grad_nan_scan(g.numel(), _lib.ptr(g), _lib.ptr(flag), st), "gf_grad_nan_scan")
         self.last_nan_flag = flag
         return flag
+
+    def _nan_flags(self, grads):
+        """device int32 [len(grads)]: flag k = any NaN in grads[k] (one guard per focal block); None when the guard is
+        off"""
+        if not self.nan_guard:
+            return None
+        flags = self._buf("nan_flags", (len(grads),), torch.int32, zero=True)
+        L, st = _lib.lib(), _lib.cur_stream()
+        for k, g in enumerate(grads):
+            _lib.check(L.gf_grad_nan_scan(g.numel(), _lib.ptr(g), _lib.ptr(flags[k:]), st), "gf_grad_nan_scan")
+        self.last_nan_flag = flags
+        return flags
 
     def _apply_adam(self, lr_scale: float):
         div = float(self.world)

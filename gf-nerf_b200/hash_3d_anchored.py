@@ -213,6 +213,43 @@ class Hash3DAnchoredCore:
                 _lib.ptr(ray_id), _lib.ptr(ray_table), _lib.ptr(base_f16), _lib.ptr(out_f16), _lib.cur_stream()),
                 "gf_hash_forward_residual_routed")
 
+    @staticmethod
+    def grad_refs(cores, grads, device) -> torch.Tensor:
+        """The gf_hash_grad_ref array of `cores` on `device` (int64 [K, 3]: prime pool, bias pool or 0, gradient
+        table), for `launch_backward_routed`.  grads[k]: fp32 [pool_size, 2] gradient table of cores[k].  It holds
+        addresses: valid until a pool or gradient table is reallocated.  The bias-pool tests may read the host."""
+        cores, grads = list(cores), list(grads)
+        if not cores or len(cores) != len(grads):
+            raise ValueError(f"Hash3DAnchored routed scatter: {len(cores)} tables and {len(grads)} gradient tables")
+        c0 = cores[0]
+        for c, g in zip(cores, grads):
+            if c.local_size_ != c0.local_size_ or c.n_volumes_ != c0.n_volumes_:
+                raise ValueError(f"Hash3DAnchored routed scatter: tables of local_size / n_volumes {c.local_size_} / "
+                                 f"{c.n_volumes_} and {c0.local_size_} / {c0.n_volumes_}; all must agree")
+            if g.dtype != torch.float32 or not g.is_contiguous() or g.numel() != c.pool_size_ * N_CHANNELS:
+                raise ValueError("Hash3DAnchored routed scatter: each gradient table is a contiguous fp32 tensor of "
+                                 "its table's size")
+        rows = [[c.prim_pool_.data_ptr(), _lib.ptr(c._bias()) or 0, g.data_ptr()] for c, g in zip(cores, grads)]
+        return torch.tensor(rows, dtype=torch.int64).to(device, non_blocking=True)
+
+    @staticmethod
+    def launch_backward_routed(cores, points, anchors, grad_in, grad_is_scaled_f16, ray_id, ray_table, grads=None,
+                               refs=None, d_n_ptr=None, keep_x128=False):
+        """`launch_backward` with one gradient table per sample: sample i accumulates into grads[ray_table[ray_id[i]]]
+        with that table's pools, what `launch_backward` of cores[k] into grads[k] computes for it; a table id outside
+        [0, len(cores)) contributes nothing.  refs: `grad_refs(cores, grads, ...)` made once by a caller that launches
+        many times (else built here from `grads`, one host-to-device copy)."""
+        assert ray_id.dtype == torch.int32 and ray_table.dtype == torch.int32
+        if refs is None:
+            refs = Hash3DAnchoredCore.grad_refs(cores, grads, points.device)
+        c0 = cores[0]
+        with torch.cuda.device(points.device):
+            _lib.check(_lib.lib().gf_hash_backward_routed(
+                points.shape[0], _lib.ptr(d_n_ptr), c0.n_volumes_, c0.local_size_, len(cores), _lib.ptr(refs),
+                _lib.ptr(c0.level_scales_), _lib.ptr(points), _lib.ptr(anchors), int(anchors.dtype == torch.int64),
+                _lib.ptr(ray_id), _lib.ptr(ray_table), _lib.ptr(grad_in),
+                int(bool(grad_is_scaled_f16)) | (2 if keep_x128 else 0), _lib.cur_stream()), "gf_hash_backward_routed")
+
     def launch_backward(self, points, anchors, grad_in, grad_is_scaled_f16, grad_table, d_n_ptr=None,
                         keep_x128=False, levels=(0, 16)):
         """keep_x128: leave grad_table at the reference's x128 gradient scale (Hash3DAnchored_cuda.cu:209) for a

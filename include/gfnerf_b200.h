@@ -134,6 +134,25 @@ int gf_hash_backward_levels(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes
                             const void* grad_in, int grad_in_is_scaled_f16,
                             float* grad_table, int level_begin, int level_end, void* stream);
 
+/* One gradient table of gf_hash_backward_routed: the prime pool and bias pool (NULL = zeros) the forward used, and the
+ * fp32 gradient table [n_levels*local_size, 2] the table's samples accumulate into. */
+typedef struct {
+  const int32_t* prim_pool;
+  const float* bias_pool;
+  float* grad_table;
+} gf_hash_grad_ref;
+
+/* gf_hash_backward_levels (all 16 levels) with one of n_tables gradient tables per sample: sample i accumulates into
+ * table t = ray_table[ray_id[i]] of d_tables (a DEVICE array of n_tables descriptors) exactly what
+ * gf_hash_backward_levels with table t's prime / bias pools and grad_table computes for it; a t outside [0, n_tables)
+ * contributes nothing.  All tables share local_size and n_volumes; grad_in and its flags as gf_hash_backward.  Runs of
+ * samples are summed only within one table.  The focal stage trains several blocks in one step: each ray's samples
+ * go to its block's table in one launch. */
+int gf_hash_backward_routed(int64_t n, const int32_t* d_n_ptr, int32_t n_volumes, int64_t local_size,
+                            int32_t n_tables, const gf_hash_grad_ref* d_tables, const float* level_scales,
+                            const float* pts, const void* anchors, int anchor_i64, const int32_t* ray_id,
+                            const int32_t* ray_table, const void* grad_in, int grad_in_is_scaled_f16, void* stream);
+
 /* Parity probe: rows int32 [n,16,8] = table row (level offset included) of the 8 corners of
  * every (point, level), order 000,001,...,111 (:48-55).  Not on the hot path. */
 int gf_hash_corner_rows(int64_t n, int32_t n_volumes, int64_t local_size, const int32_t* prim_pool,
